@@ -1,7 +1,11 @@
 #!/usr/bin/env python
 """Headline benchmark: images/sec of the static-PTQ int8 SimpleConvNet forward (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
+
+``--dump-outputs DIR`` writes the logits of the last timed step as ``DIR/logits.npy`` (float32; ``logits_rank<r>.npy``
+for ranks > 0), so two builds of the project can be compared output for output: inputs and weights are generated from
+fixed seeds, so the same arguments give the same inputs on every run.
 
 * ours (default): one process per GPU (torchrun for N>1).  A step = one ``b200q_static_forward`` over a batch of
   B synthetic images resident in HBM (fp32 NCHW, the reference's input contract).  ``value`` = all ranks' images /
@@ -154,13 +158,13 @@ def time_cpu_oracle(q, batch: int, batches_per_step: int, steps: int, warmup: in
     x = synth.images_f32(batch, seed=11)
     with torch.no_grad():
         for _ in range(max(1, warmup)):
-            q(x)
+            y = q(x)
         t0 = time.perf_counter()
         for _ in range(steps):
             for _ in range(batches_per_step):
-                q(x)
+                y = q(x)
         dt = time.perf_counter() - t0
-    return batch * batches_per_step * steps / dt, dt, cores
+    return batch * batches_per_step * steps / dt, dt, cores, y
 
 
 def run_reference(args):
@@ -169,7 +173,9 @@ def run_reference(args):
         return 0
     q = build_cpu_oracle()
     batch, per_step = 64, 16  # BASELINE config 1: batch 64 on CPU; a step = 16 such batches (1024 images)
-    ips, dt, cores = time_cpu_oracle(q, batch, per_step, args.steps, args.warmup)
+    ips, dt, cores, y = time_cpu_oracle(q, batch, per_step, args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits": y})
     sample = f"{args.steps} steps x {per_step} batches x {batch} images (torch {torch.__version__} fbgemm, {cores} threads)"
     line = {
         "impl": "reference", "metric": METRIC, "value": ips, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -210,6 +216,25 @@ def ncu_traffic(stage: str, batch: int):
         except (OSError, KeyError, ValueError, TypeError):
             continue
     return None
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Write each tensor of ``arrays`` as ``out_dir/<name>.npy`` (float32 or float64).  A tensor larger than 64 MB is
+    cut to a fixed, seeded sample of its rows, kept in their original order."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().cpu()
+        if a.dtype not in (torch.float32, torch.float64):
+            a = a.float()
+        nbytes = a.numel() * a.element_size()
+        if nbytes > DUMP_MAX_BYTES:
+            keep = DUMP_MAX_BYTES * a.shape[0] // nbytes
+            a = a[torch.randperm(a.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values]
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a.numpy()))
 
 
 def oracle_sample_indices(n: int, count: int = 1024):
@@ -285,6 +310,8 @@ def run_ours(args):
     launches = int(lib.b200q_launch_count() - n0)
     ms = max_over_ranks(ev0.elapsed_time(ev1))
     value = world * B * args.steps / (ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"logits" if rank == 0 else f"logits_rank{rank}": logits})
 
     # ---- per-kernel durations of the same forward (CUDA events between kernels, on the launching stream)
     prof_steps = max(3, min(args.steps, 20))
@@ -416,9 +443,9 @@ def run_ours(args):
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         q = q_oracle if parity is not None else build_cpu_oracle()
         # bounded sample: ~10-20 s of CPU work at batch 64 (BASELINE config 1)
-        ips0, _, cores = time_cpu_oracle(q, 64, 8, 2, 1)
+        ips0, _, cores, _ = time_cpu_oracle(q, 64, 8, 2, 1)
         steps_cpu = max(2, int(12.0 * ips0 / (64 * 16)))
-        ips, dt, cores = time_cpu_oracle(q, 64, 16, steps_cpu, 1)
+        ips, dt, cores, _ = time_cpu_oracle(q, 64, 16, steps_cpu, 1)
         cpu_baseline = {"value": ips, "unit": UNIT, "cores": cores, "kind": "port",
                         "sample": f"{steps_cpu * 16} batches x 64 images in {dt:.1f} s, torch {torch.__version__} "
                                   f"fbgemm static-PTQ oracle, {cores} threads"}
@@ -512,6 +539,8 @@ def run_variant(args):
         ms = ev0.elapsed_time(ev1)
         launches = int(lib.b200q_launch_count() - n0)
         value = B * args.steps / (ms * 1e-3)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"logits": y})
 
         x_host = x.cpu().pin_memory()
         e2e_steps = max(3, min(args.steps, 20))
@@ -601,7 +630,11 @@ def main():
     ap.add_argument("--variant", default="static", choices=["static", "dynamic", "fp32", "custom", "custom_sandwich"],
                     help="static = the headline (BASELINE config 2/5); the others are BASELINE configs 3-4")
     ap.add_argument("--stages-only", action="store_true", help="print only the per-kernel table (timing experiments)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the logits of the last timed step to DIR/logits.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "ours" and world != args.gpus and args.gpus > 1:
         raise SystemExit(f"--gpus {args.gpus} needs torchrun with {args.gpus} ranks (WORLD_SIZE={world})")

@@ -1,18 +1,17 @@
 """The drop-in view (SURVEY 8d): the reference's OWN, unmodified `utils/inference_benchmark.py` timing this package's
 models on the GPU (`device='cuda'`) next to the torch/fbgemm CPU oracle model on the host (`device='cpu'`), at the
 driver's own operating points (batch 1 and batch 32, `inference_benchmark.py:126-138`).
-    python scripts/reference_driver_view.py > profiles/r02_reference_driver_view.json
-Needs the two driver files under /root/reference or baseline/_ref (staged by `__graft_entry__.build()`)."""
+    python scripts/reference_driver_view.py REFERENCE_CHECKOUT > profiles/r02_reference_driver_view.json
+REFERENCE_CHECKOUT is a checkout of the reference project (the driver is imported from its `utils/`)."""
 import contextlib, io, json, os, sys, warnings
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 warnings.filterwarnings("ignore")
 import torch
 
-ref_root = next((c for c in ("/root/reference", os.path.join(ROOT, "baseline", "_ref"))
-                 if os.path.isfile(os.path.join(c, "utils", "inference_benchmark.py"))), None)
-if ref_root is None:
-    raise SystemExit("reference drivers not found")
+ref_root = sys.argv[1] if len(sys.argv) > 1 else ""
+if not os.path.isfile(os.path.join(ref_root, "utils", "inference_benchmark.py")):
+    raise SystemExit("usage: reference_driver_view.py REFERENCE_CHECKOUT (no utils/inference_benchmark.py there)")
 sys.path.insert(0, ref_root)
 from utils.inference_benchmark import InferenceBenchmark  # noqa: E402  (the reference's file, unmodified)
 

@@ -1,9 +1,6 @@
 """The drop-in surface (SURVEY 8b) without a GPU: class names, methods, attributes and the pre-``quantize()`` behaviour of
-the model classes mirror the reference's (`models/*.py`); when /root/reference is importable the lists are taken from
-its own classes."""
+the model classes mirror the reference's (`models/*.py`, as listed in SURVEY.md 8(b))."""
 import inspect
-import os
-import sys
 
 import pytest
 import torch
@@ -62,28 +59,3 @@ def test_behaviour_before_quantize_is_the_fp32_net():
     with pytest.raises(ValueError):
         CustomQuantizationModel(mode="nope")
 
-
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="reference tree not present")
-def test_surface_matches_the_reference_classes():
-    saved = list(sys.path)
-    mods = {k: v for k, v in sys.modules.items() if k == "models" or k.startswith("models.")}
-    for k in mods:
-        del sys.modules[k]
-    sys.path.insert(0, "/root/reference")
-    try:
-        from models.custom_quantization_model import CustomQuantizationModel as RC
-        from models.dynamic_ptq_model import DynamicPTQModel as RD
-        from models.static_ptq_model import StaticPTQModel as RS
-        for ref, ours in ((RD, DynamicPTQModel), (RS, StaticPTQModel), (RC, CustomQuantizationModel)):
-            ref_public = {n for n, v in vars(ref).items() if callable(v) and (not n.startswith("_") or n in ("__call__",))}
-            missing = {n for n in ref_public if not callable(getattr(ours, n, None))}
-            assert not missing, f"{ours.__name__} lacks {missing}"
-            for n in ref_public & {"quantize", "get_model_size", "load_state_dict", "to"}:
-                want = [p for p in inspect.signature(getattr(ref, n)).parameters]
-                got = [p for p in inspect.signature(getattr(ours, n)).parameters]
-                assert got[:len(want)] == want, f"{ours.__name__}.{n}: {got} vs reference {want}"
-    finally:
-        sys.path[:] = saved
-        for k in [k for k in sys.modules if k == "models" or k.startswith("models.")]:
-            del sys.modules[k]
-        sys.modules.update(mods)
