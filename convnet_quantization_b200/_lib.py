@@ -34,7 +34,7 @@ EXPORTS = (
     "b200q_lut_u8", "b200q_conv3x3_first", "b200q_quantize_conv3x3_first", "b200q_u8_conv3x3_first", "b200q_conv3x3_tc",
     "b200q_linear_tc", "b200q_linear_simt", "b200q_linear_dequant", "b200q_linear_dynamic",
     "b200q_static_workspace_bytes", "b200q_static_forward", "b200q_static_forward_u8", "b200q_graph_create",
-    "b200q_graph_launch", "b200q_graph_destroy", "b200q_static_num_stages", "b200q_static_stage_name",
+    "b200q_graph_create_u8", "b200q_graph_launch", "b200q_graph_destroy", "b200q_static_num_stages", "b200q_static_stage_name",
     "b200q_static_forward_profiled",
 )
 DEV_EXPORTS = EXPORTS + ("b200q_conv12_fused", "b200q_conv3x3_simt")
@@ -132,6 +132,7 @@ _SIGNATURES = {
     "b200q_histc": [_P, _L, _F, _F, _I, _P, _P],
     "b200q_lut_u8": [_P, _P, _L, _P, _P],
     "b200q_graph_create": [C.POINTER(StaticNet), _P, _P, _L, _P, _L, _I, _P, C.POINTER(C.c_void_p)],
+    "b200q_graph_create_u8": [C.POINTER(StaticNet), _P, _P, _P, _L, _P, _L, _I, _P, C.POINTER(C.c_void_p)],
     "b200q_graph_launch": [_P, _P],
     "b200q_graph_destroy": [_P],
     "b200q_conv3x3_first": [_P, _P, _L, C.POINTER(Conv3x3), _P],

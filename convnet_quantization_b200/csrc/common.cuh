@@ -28,10 +28,19 @@ int num_sms();
 // cudaFuncAttributeMaxDynamicSharedMemorySize is a PER-DEVICE attribute: `mask` (one static per kernel instantiation)
 // remembers on which devices of this process it has been raised for `kernel`.
 int ensure_dynamic_smem(const void* kernel, int bytes, uint64_t* mask);
+// uint8 input path (SURVEY 8f rank 4): raw uint8 NHWC pixels [b,32,32,3] go through a per-channel 256-entry table
+// lut[c][v] = quantize_per_tensor(Normalize(ToTensor(v))) that the host builds with the reference's own torch CPU ops,
+// so the result is bit-identical to quantising the fp32 tensor the reference's DataLoader would have produced.  The
+// first-layer kernels (conv1_tc.cu, simt.cu) take it by value as a kernel parameter.
+struct C1Lut {
+  uint8_t q[3][256];
+};
+
 // conv_halo.cu: halo-resident kernel for the cin=64 layers; returns 1 when the geometry is not covered
-// conv1_tc.cu: tensor-core first layer (fused quantize); returns 1 when the layer cannot take that path
-int conv1_tc_dispatch(const float* x, uint8_t* y, int64_t b, float inv_scale, const b200q_conv3x3* L, cudaStream_t s,
-                      int* rc);
+// conv1_tc.cu: tensor-core first layer, fp32 NCHW x with the fused quantiser or (lut_host != nullptr, a HOST
+// uint8[3][256] table) uint8 NHWC xu8; returns 1 when the layer cannot take that path
+int conv1_tc_dispatch(const float* x, const uint8_t* xu8, const uint8_t* lut_host, uint8_t* y, int64_t b,
+                      float inv_scale, const b200q_conv3x3* L, cudaStream_t s, int* rc);
 int conv3x3_halo_dispatch(const uint8_t* x, uint8_t* y, int64_t b, const b200q_conv3x3* L, bool pool, cudaStream_t s,
                           int* rc);
 // conv_halo2.cu: conv2 + fused pool on CTA pairs (tcgen05.mma.cta_group::2); returns 1 when not covered

@@ -39,13 +39,6 @@ constexpr int C1_Q_BYTES = (C1_QP * C1_QP * 4 + 15) / 16 * 16;
 constexpr int C1_LUT_BYTES = 3 * 256;
 constexpr int C1_SMEM = 2 * C1_A_BYTES + C1_B_BYTES + C1_Q_BYTES + 256 + C1_LUT_BYTES + 1024;
 
-// uint8 input path (SURVEY 8f rank 4): raw uint8 NHWC pixels [b,32,32,3] go through a per-channel 256-entry table
-// lut[c][v] = quantize_per_tensor(Normalize(ToTensor(v))) that the host builds with the reference's own torch CPU ops,
-// so the result is bit-identical to quantising the fp32 tensor the reference's DataLoader would have produced.
-struct C1Lut {
-  uint8_t q[3][256];
-};
-
 struct C1Args {
   const float* x;
   const uint8_t* xu8;  // uint8 NHWC [b,32,32,3] (U8IN kernels), else null
@@ -290,8 +283,9 @@ conv1_tc_kernel(const __grid_constant__ C1Consts consts, const __grid_constant__
 }
 
 // x: fp32 NCHW input (lut_host == nullptr) or, with lut_host = uint8[3][256] on the HOST, xu8: uint8 NHWC input.
-static int conv1_tc_launch(const float* x, const uint8_t* xu8, const uint8_t* lut_host, uint8_t* y, int64_t b, float inv_scale,
-                           const b200q_conv3x3* L, cudaStream_t s, int* rc) {
+// Returns 1 when the layer cannot take this path (no host mirrors / constants not flagged as bounded).
+int conv1_tc_dispatch(const float* x, const uint8_t* xu8, const uint8_t* lut_host, uint8_t* y, int64_t b,
+                      float inv_scale, const b200q_conv3x3* L, cudaStream_t s, int* rc) {
   const b200q_requant& rq = L->rq;
   if (!L->corr_host || !rq.mult_host || !rq.bdiv_host || !(rq.flags & B200Q_RQ_BOUNDED)) return 1;
   if (L->cin != 4 || L->cout != C1_COUT || L->img != C1_IMG) return 1;
@@ -323,26 +317,5 @@ static int conv1_tc_launch(const float* x, const uint8_t* xu8, const uint8_t* lu
   return 0;
 }
 
-// Returns 1 when the layer cannot take this path (no host mirrors / constants not flagged as bounded).
-int conv1_tc_dispatch(const float* x, uint8_t* y, int64_t b, float inv_scale, const b200q_conv3x3* L, cudaStream_t s,
-                      int* rc) {
-  return conv1_tc_launch(x, nullptr, nullptr, y, b, inv_scale, L, s, rc);
-}
-
 }  // namespace b200q
-
-using namespace b200q;
-
-extern "C" int b200q_u8_conv3x3_first(const uint8_t* x_nhwc, uint8_t* y, int64_t b, const uint8_t* lut_host,
-                                      const b200q_conv3x3* L, void* stream) {
-  B200Q_REQUIRE(L && lut_host && ((x_nhwc && y) || b == 0), "u8_conv3x3_first: null pointer");
-  B200Q_REQUIRE((uintptr_t)x_nhwc % 8 == 0 && (uintptr_t)y % 16 == 0, "u8_conv3x3_first: misaligned buffers");
-  if (b == 0) return 0;
-  int rc = 0;
-  if (conv1_tc_launch(nullptr, x_nhwc, lut_host, y, b, 0.f, L, (cudaStream_t)stream, &rc) != 0) {
-    set_error("u8_conv3x3_first: layer must be conv1 (cin 4, cout 64, img 32) with host mirrors and B200Q_RQ_BOUNDED");
-    return B200Q_ERR_INVALID_ARG;
-  }
-  return rc;
-}
 

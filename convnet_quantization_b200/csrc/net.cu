@@ -197,16 +197,20 @@ struct b200q_graph {
   int kernels = 0;  // kernels one replay launches (b200q_launch_count bookkeeping)
 };
 
-extern "C" int b200q_graph_create(const b200q_static_net* net, const float* x_static, float* logits_static, int64_t b,
-                                  void* workspace, int64_t workspace_bytes, int flags, void* stream, b200q_graph** out) {
+namespace {
+// One capture body for both input kinds: x (fp32 NCHW) or x_u8 + lut_host (uint8 NHWC pixels, HOST table).
+int graph_create_impl(const b200q_static_net* net, const float* x, const uint8_t* x_u8, const uint8_t* lut_host,
+                      float* logits_static, int64_t b, void* workspace, int64_t workspace_bytes, int flags, void* stream,
+                      b200q_graph** out) {
   B200Q_REQUIRE(out != nullptr, "graph_create: null out");
   *out = nullptr;
-  B200Q_REQUIRE(net && x_static && logits_static && workspace && b > 0, "graph_create: null pointer or empty batch");
+  B200Q_REQUIRE(net && (x || (x_u8 && lut_host)) && logits_static && workspace && b > 0,
+                "graph_create: null pointer or empty batch");
   B200Q_REQUIRE(stream != nullptr, "graph_create: the legacy default stream cannot be captured; pass a created stream");
   cudaStream_t s = (cudaStream_t)stream;
   // eager first: per-device kernel attributes, lazy module loading and the tensor-map encoder are first-use work that
   // does not belong inside a capture
-  int rc = forward_impl(net, x_static, logits_static, b, workspace, workspace_bytes, nullptr, nullptr, stream);
+  int rc = forward_impl(net, x, logits_static, b, workspace, workspace_bytes, nullptr, nullptr, stream, x_u8, lut_host);
   if (rc) return rc;
   B200Q_CUDA(cudaStreamSynchronize(s));  // (the eager forward above left the head kernel's ticket word zero)
   B200Q_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
@@ -215,7 +219,7 @@ extern "C" int b200q_graph_create(const b200q_static_net* net, const float* x_st
   g_stop_after = (flags >> 8) & 15;  // development library: capture only the first k kernels (timing breakdown)
 #endif
   const uint64_t launches0 = b200q_launch_count();
-  rc = forward_impl(net, x_static, logits_static, b, workspace, workspace_bytes, nullptr, nullptr, stream, nullptr, nullptr,
+  rc = forward_impl(net, x, logits_static, b, workspace, workspace_bytes, nullptr, nullptr, stream, x_u8, lut_host,
                     /*ticket_is_zero=*/true);
   const int captured_kernels = (int)(b200q_launch_count() - launches0);
   pdl_set(false);
@@ -246,6 +250,20 @@ extern "C" int b200q_graph_create(const b200q_static_net* net, const float* x_st
   }
   *out = g;
   return 0;
+}
+}  // namespace
+
+extern "C" int b200q_graph_create(const b200q_static_net* net, const float* x_static, float* logits_static, int64_t b,
+                                  void* workspace, int64_t workspace_bytes, int flags, void* stream, b200q_graph** out) {
+  return graph_create_impl(net, x_static, nullptr, nullptr, logits_static, b, workspace, workspace_bytes, flags, stream,
+                           out);
+}
+
+extern "C" int b200q_graph_create_u8(const b200q_static_net* net, const uint8_t* x_nhwc_static, const uint8_t* lut_host,
+                                     float* logits_static, int64_t b, void* workspace, int64_t workspace_bytes, int flags,
+                                     void* stream, b200q_graph** out) {
+  return graph_create_impl(net, nullptr, x_nhwc_static, lut_host, logits_static, b, workspace, workspace_bytes, flags,
+                           stream, out);
 }
 
 extern "C" int b200q_graph_launch(b200q_graph* g, void* stream) {

@@ -6,7 +6,12 @@
 namespace b200q {
 
 // =========================================================================================================
-// First conv (cin = 3 stored as 4, cout = 64, 32x32 images), optionally fused with aten::quantize_per_tensor.
+// First conv (cin = 3 stored as 4, cout = 64, 32x32 images).  Input kinds (C1In):
+//   C1_IN_NHWC4  uint8 NHWC4, already quantised (b200q_conv3x3_first);
+//   C1_IN_F32    fp32 NCHW, fused with aten::quantize_per_tensor (b200q_quantize_conv3x3_first);
+//   C1_IN_U8     raw uint8 NHWC pixels [b,32,32,3] through the host table C1Lut (b200q_u8_conv3x3_first): the halo word
+//                lut[0][p0] | lut[1][p1]<<8 | lut[2][p2]<<16 | zp_x<<24 is the word C1_IN_F32 builds from the
+//                normalised pixels, and everything after the halo load is shared, so the two agree bit for bit.
 // Block = 8 output rows x 32 columns of one image (256 threads, one pixel each, all 64 output channels).
 // The quantized halo (10 x 34 pixels, one 32-bit word per pixel) lives in shared memory; out-of-image taps hold
 // zp_x (real-domain zero), so acc_true = sum_all x*w - zp_x*sum_all w = raw - corr[interior][c] for every pixel.
@@ -18,16 +23,20 @@ constexpr int C1_ROWS = 8;
 constexpr int C1_COUT = 64;
 constexpr int CONV1_TINY_MAX_B = 32;  // measured: ahead of conv1_tc.cu up to 32 images, level at 64 (r02 sweep)
 
-template <bool FUSED_QUANT, int CGROUPS>
+enum C1In { C1_IN_NHWC4 = 0, C1_IN_F32 = 1, C1_IN_U8 = 2 };
+
+template <int IN, int CGROUPS>
 __global__ void __launch_bounds__(256) conv1_kernel(const void* __restrict__ xin, uint8_t* __restrict__ y,
                                                     const uint32_t* __restrict__ w_words,  // [64][9] words
                                                     const int32_t* __restrict__ corr,      // [9][64], row 4 = interior
                                                     const float* __restrict__ mult, const float* __restrict__ bdiv,
-                                                    int zp_x, int zp_out, int relu, float inv_scale, int img) {
+                                                    int zp_x, int zp_out, int relu, float inv_scale, int img,
+                                                    const __grid_constant__ C1Lut lut) {  // read by C1_IN_U8 only
   __shared__ uint32_t s_in[(C1_ROWS + 2) * 34];
   __shared__ uint4 s_w[9 * (C1_COUT / 4)];
   __shared__ float s_mult[C1_COUT], s_bdiv[C1_COUT];
   __shared__ int s_corr[C1_COUT];
+  __shared__ uint32_t s_lut[IN == C1_IN_U8 ? 3 * 256 / 4 : 1];  // [3][256] bytes
 
   const int tiles_per_img = img / C1_ROWS;
   const int64_t image = blockIdx.x / tiles_per_img;
@@ -46,17 +55,26 @@ __global__ void __launch_bounds__(256) conv1_kernel(const void* __restrict__ xin
     s_bdiv[tid] = __ldg(bdiv + tid);
     s_corr[tid] = __ldg(corr + 4 * C1_COUT + tid);
   }
+  if constexpr (IN == C1_IN_U8) {  // the table is a kernel parameter, not the previous kernel's output
+    if (tid < 3 * 256 / 4) s_lut[tid] = reinterpret_cast<const uint32_t*>(&lut.q[0][0])[tid];
+    __syncthreads();
+  }
   pdl_wait();  // y may still be read by the previous kernel of the stream (weights and constants above are not its output)
   for (int i = tid; i < (C1_ROWS + 2) * 34; i += 256) {
     const int r = i / 34 + row0 - 1, c = i % 34 - 1;
     uint32_t word = zp_word;
     if (r >= 0 && r < img && c >= 0 && c < img) {
-      if constexpr (FUSED_QUANT) {
+      if constexpr (IN == C1_IN_F32) {
         const float* x = reinterpret_cast<const float*>(xin) + image * 3 * img * img + r * img + c;
         const uint32_t q0 = quantize_u8(__ldg(x), inv_scale, zp_x);
         const uint32_t q1 = quantize_u8(__ldg(x + img * img), inv_scale, zp_x);
         const uint32_t q2 = quantize_u8(__ldg(x + 2 * img * img), inv_scale, zp_x);
         word = q0 | (q1 << 8) | (q2 << 16) | ((uint32_t)zp_x << 24);
+      } else if constexpr (IN == C1_IN_U8) {
+        const uint8_t* p = reinterpret_cast<const uint8_t*>(xin) + ((image * img + r) * img + c) * 3;
+        const uint8_t* t = reinterpret_cast<const uint8_t*>(s_lut);
+        word = (uint32_t)t[__ldg(p)] | ((uint32_t)t[256 + __ldg(p + 1)] << 8) | ((uint32_t)t[512 + __ldg(p + 2)] << 16) |
+               ((uint32_t)zp_x << 24);
       } else {
         word = __ldg(reinterpret_cast<const uint32_t*>(xin) + (image * img + r) * img + c);
       }
@@ -414,16 +432,26 @@ static int conv1_tiny_max_b() {
   return v;
 }
 
-static int conv_first_impl(const void* x, uint8_t* y, int64_t b, const b200q_conv3x3* L, bool fused, float inv_scale,
-                           void* stream) {
+// kind: C1_IN_NHWC4 (x uint8 NHWC4), C1_IN_F32 (x fp32 NCHW, inv_scale) or C1_IN_U8 (x uint8 NHWC pixels, lut_host a HOST
+// uint8[3][256] table).  The two raw-input kinds share the kernel selection: the CUDA-core shape for a few images, else
+// the tensor-core kernel, else (layer without host mirrors / BOUNDED constants) the CUDA-core kernel for any batch.
+static int conv_first_impl(const void* x, uint8_t* y, int64_t b, const b200q_conv3x3* L, C1In kind, float inv_scale,
+                           const uint8_t* lut_host, void* stream) {
   int rc = check_conv(x, y, b, L);
   if (rc) return rc;
   B200Q_REQUIRE(L->cin == 4 && L->cout == C1_COUT && L->img == 32,
                 "conv3x3_first: geometry must be cin=3(padded 4), cout=64, img=32 (got %d,%d,%d)", L->cin, L->cout,
                 L->img);
-  B200Q_REQUIRE((uintptr_t)y % 16 == 0 && (uintptr_t)x % 4 == 0, "conv3x3_first: misaligned buffers");
+  B200Q_REQUIRE((uintptr_t)y % 16 == 0 && (uintptr_t)x % (kind == C1_IN_U8 ? 8 : 4) == 0,
+                "conv3x3_first: misaligned buffers");
   if (b == 0) return 0;
-  if (fused && b <= conv1_tiny_max_b()) {  // a few images: 16 CUDA-core CTAs per image, one round trip
+  static const C1Lut kNoLut = {};
+  C1Lut lut;
+  if (kind == C1_IN_U8)
+    for (int i = 0; i < 3 * 256; ++i) lut.q[i / 256][i % 256] = lut_host[i];
+  const C1Lut& lut_arg = kind == C1_IN_U8 ? lut : kNoLut;
+  const bool raw = kind != C1_IN_NHWC4;
+  if (raw && b <= conv1_tiny_max_b()) {  // a few images: 16 CUDA-core CTAs per image, one round trip
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)(b * (L->img / C1_ROWS)), 4);
     cfg.blockDim = dim3(256);
@@ -435,16 +463,17 @@ static int conv_first_impl(const void* x, uint8_t* y, int64_t b, const b200q_con
       cfg.attrs = attr;
       cfg.numAttrs = 1;
     }
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, conv1_kernel<true, 1>, x, y, reinterpret_cast<const uint32_t*>(L->w),
-                                             L->corr, L->rq.mult, L->rq.bdiv, (int)L->zp_x, (int)L->rq.zp_out,
-                                             (int)L->rq.relu, inv_scale, (int)L->img);
+    const cudaError_t e = cudaLaunchKernelEx(
+        &cfg, kind == C1_IN_U8 ? conv1_kernel<C1_IN_U8, 1> : conv1_kernel<C1_IN_F32, 1>, x, y,
+        reinterpret_cast<const uint32_t*>(L->w), L->corr, L->rq.mult, L->rq.bdiv, (int)L->zp_x, (int)L->rq.zp_out,
+        (int)L->rq.relu, inv_scale, (int)L->img, lut_arg);
     if (e != cudaSuccess) {
       (void)cudaGetLastError();
       return check_cuda(e, "conv1_kernel");
     }
     return launched("conv1_kernel");
   }
-  if (fused) {  // tensor-core version unless the layer lacks host mirrors / the BOUNDED flag (dev builds: or B200Q_NO_CONV1_TC=1)
+  if (raw) {  // tensor-core version unless the layer lacks host mirrors / the BOUNDED flag (dev builds: or B200Q_NO_CONV1_TC=1)
 #ifdef B200Q_DEV
     static int no_tc = -1;
     if (no_tc < 0) {
@@ -455,27 +484,36 @@ static int conv_first_impl(const void* x, uint8_t* y, int64_t b, const b200q_con
     const int no_tc = 0;
 #endif
     int trc = 0;
-    if (!no_tc && conv1_tc_dispatch(reinterpret_cast<const float*>(x), y, b, inv_scale, L, (cudaStream_t)stream, &trc) == 0)
+    const bool u8 = kind == C1_IN_U8;
+    if (!no_tc && conv1_tc_dispatch(u8 ? nullptr : reinterpret_cast<const float*>(x),
+                                    u8 ? reinterpret_cast<const uint8_t*>(x) : nullptr, u8 ? lut_host : nullptr, y, b,
+                                    inv_scale, L, (cudaStream_t)stream, &trc) == 0)
       return trc;
   }
   const unsigned grid = (unsigned)(b * (L->img / C1_ROWS));
   const uint32_t* ww = reinterpret_cast<const uint32_t*>(L->w);
-  if (fused)
-    conv1_kernel<true, 4><<<grid, 256, 0, (cudaStream_t)stream>>>(x, y, ww, L->corr, L->rq.mult, L->rq.bdiv, L->zp_x,
-                                                                  L->rq.zp_out, L->rq.relu, inv_scale, L->img);
-  else
-    conv1_kernel<false, 4><<<grid, 256, 0, (cudaStream_t)stream>>>(x, y, ww, L->corr, L->rq.mult, L->rq.bdiv, L->zp_x,
-                                                                   L->rq.zp_out, L->rq.relu, 0.f, L->img);
+  void (*kernel)(const void*, uint8_t*, const uint32_t*, const int32_t*, const float*, const float*, int, int, int, float,
+                 int, C1Lut) = kind == C1_IN_U8    ? conv1_kernel<C1_IN_U8, 4>
+                               : kind == C1_IN_F32 ? conv1_kernel<C1_IN_F32, 4>
+                                                   : conv1_kernel<C1_IN_NHWC4, 4>;
+  kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(x, y, ww, L->corr, L->rq.mult, L->rq.bdiv, L->zp_x, L->rq.zp_out,
+                                                 L->rq.relu, kind == C1_IN_F32 ? inv_scale : 0.f, L->img, lut_arg);
   return launched("conv1_kernel");
 }
 
 extern "C" int b200q_conv3x3_first(const uint8_t* x, uint8_t* y, int64_t b, const b200q_conv3x3* L, void* stream) {
-  return conv_first_impl(x, y, b, L, false, 0.f, stream);
+  return conv_first_impl(x, y, b, L, C1_IN_NHWC4, 0.f, nullptr, stream);
 }
 
 extern "C" int b200q_quantize_conv3x3_first(const float* x, uint8_t* y, int64_t b, float inv_scale,
                                             const b200q_conv3x3* L, void* stream) {
-  return conv_first_impl(x, y, b, L, true, inv_scale, stream);
+  return conv_first_impl(x, y, b, L, C1_IN_F32, inv_scale, nullptr, stream);
+}
+
+extern "C" int b200q_u8_conv3x3_first(const uint8_t* x_nhwc, uint8_t* y, int64_t b, const uint8_t* lut_host,
+                                      const b200q_conv3x3* L, void* stream) {
+  B200Q_REQUIRE(lut_host != nullptr, "u8_conv3x3_first: null lut_host");
+  return conv_first_impl(x_nhwc, y, b, L, C1_IN_U8, 0.f, lut_host, stream);
 }
 
 #ifdef B200Q_DEV

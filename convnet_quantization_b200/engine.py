@@ -31,9 +31,10 @@ def _current_stream_handle(device_index: int) -> int:
 
 
 class _Graph:
-    """One captured forward (``b200q_graph_*``): fixed batch, fixed input / logits buffers, private workspace."""
+    """One captured forward (``b200q_graph_*``): fixed batch, fixed input / logits buffers, private workspace.
+    ``u8``: ``x`` holds uint8 NHWC pixels (``b200q_graph_create_u8``), else fp32 NCHW images."""
 
-    def __init__(self, engine, x: torch.Tensor, logits: torch.Tensor, pdl: bool):
+    def __init__(self, engine, x: torch.Tensor, logits: torch.Tensor, pdl: bool, u8: bool = False):
         lib = engine.lib
         b = x.shape[0]
         self.x, self.logits = x, logits  # keeps the captured buffers alive
@@ -43,9 +44,15 @@ class _Graph:
         cur = torch.cuda.current_stream(engine.device)
         side = engine._capture_stream()
         side.wait_stream(cur)
-        rc = lib.b200q_graph_create(engine.packed.ptr(), x.data_ptr(), logits.data_ptr(), b, self.ws.data_ptr(),
-                                    self.ws.numel(), _lib.GRAPH_PDL if pdl else 0, side.cuda_stream, C.byref(self.handle))
-        _lib.check(rc, "graph_create")
+        flags = _lib.GRAPH_PDL if pdl else 0
+        if u8:
+            rc = lib.b200q_graph_create_u8(engine.packed.ptr(), x.data_ptr(), engine.packed.input_lut.data_ptr(),
+                                           logits.data_ptr(), b, self.ws.data_ptr(), self.ws.numel(), flags,
+                                           side.cuda_stream, C.byref(self.handle))
+        else:
+            rc = lib.b200q_graph_create(engine.packed.ptr(), x.data_ptr(), logits.data_ptr(), b, self.ws.data_ptr(),
+                                        self.ws.numel(), flags, side.cuda_stream, C.byref(self.handle))
+        _lib.check(rc, "graph_create_u8" if u8 else "graph_create")
         cur.wait_stream(side)
 
     def launch(self, stream: int):
@@ -67,7 +74,8 @@ class StaticEngine:
     regime the reference's own driver measures (``utils/inference_benchmark.py:126-138``: batch 1 and 32) - are
     replayed from a CUDA graph captured on the caller's input buffer, with programmatic dependent launch between the
     layer kernels.  A graph is captured the second time the same (batch, input buffer[, output buffer]) is seen and
-    ``GRAPH_CACHE`` of them are kept (least recently used evicted)."""
+    ``GRAPH_CACHE`` of them are kept (least recently used evicted).  ``forward_u8`` (raw uint8 pixels) follows the
+    same policy; its graphs share the cache, keyed apart by the input kind."""
 
     GRAPH_MAX_BATCH = 1024
     GRAPH_CACHE = 8
@@ -85,7 +93,7 @@ class StaticEngine:
         with torch.cuda.device(self.device):
             self.packed = PackedStaticNet(qparams, self.device)
         self._ws = OrderedDict()      # CUDA stream handle -> workspace (forwards on different streams must not share one)
-        self._graphs = OrderedDict()  # (batch, x ptr, out ptr or 0) -> _Graph
+        self._graphs = OrderedDict()  # (uint8 input?, batch, x ptr, out ptr or 0) -> _Graph
         self._seen = OrderedDict()    # keys seen once (capture on the second sighting)
         self._side = None
 
@@ -127,9 +135,10 @@ class StaticEngine:
             raise _lib.B200QError(f"out must be a contiguous fp32 [{b},10] tensor on {self.device}, got "
                                   f"{out.dtype} {tuple(out.shape)} on {out.device}")
 
-    def _graph_for(self, x: torch.Tensor, out):
-        """The captured graph for this (batch, input buffer, output buffer), or None (not yet / not eligible)."""
-        key = (x.shape[0], x.data_ptr(), 0 if out is None else out.data_ptr())
+    def _graph_for(self, x: torch.Tensor, out, u8: bool = False):
+        """The captured graph for this (input kind, batch, input buffer, output buffer), or None (not yet / not
+        eligible)."""
+        key = (u8, x.shape[0], x.data_ptr(), 0 if out is None else out.data_ptr())
         g = self._graphs.get(key)
         if g is not None:
             self._graphs.move_to_end(key)
@@ -141,7 +150,7 @@ class StaticEngine:
             return None
         del self._seen[key]
         logits = out if out is not None else torch.empty((x.shape[0], 10), dtype=torch.float32, device=self.device)
-        g = _Graph(self, x, logits, self.pdl)
+        g = _Graph(self, x, logits, self.pdl, u8)
         self._graphs[key] = g
         while len(self._graphs) > self.GRAPH_CACHE:
             self._graphs.popitem(last=False)
@@ -191,17 +200,26 @@ class StaticEngine:
     __call__ = forward
 
     @torch.no_grad()
-    def forward_u8(self, x_u8: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
+    def forward_u8(self, x_u8: torch.Tensor, out: torch.Tensor | None = None, graph: bool | None = None) -> torch.Tensor:
         """uint8 data path: raw pixels, uint8 NHWC ``[B,32,32,3]`` (CUDA) -> fp32 logits ``[B,10]``; bit-identical to
-        ``forward(synth.normalize(pixels))`` (``packing.input_lut``)."""
+        ``forward(synth.normalize(pixels))`` (``packing.input_lut``).  ``out`` and ``graph`` as for ``forward``."""
         x_u8 = x_u8.contiguous()
         self._check_input(x_u8, (32, 32, 3), torch.uint8, "StaticEngine.forward_u8")
         b = x_u8.shape[0]
         self._check_out(out, b)
-        with torch.cuda.device(self.device):
-            logits = out if out is not None else torch.empty((b, 10), dtype=torch.float32, device=self.device)
+        ctx = _NULL_CTX if torch.cuda.current_device() == self.device.index else torch.cuda.device(self.device)
+        with ctx:
             if b == 0:
-                return logits
+                return out if out is not None else torch.empty((0, 10), dtype=torch.float32, device=self.device)
+            use_graph = self.use_graphs and b <= self.GRAPH_MAX_BATCH if graph is None else graph
+            if use_graph:
+                g = self._graph_for(x_u8, out, u8=True)
+                if g is None and graph:  # forced: capture right away
+                    g = self._graph_for(x_u8, out, u8=True)
+                if g is not None:
+                    g.launch(_current_stream_handle(self.device.index))
+                    return out if out is not None else g.logits.clone()
+            logits = out if out is not None else torch.empty((b, 10), dtype=torch.float32, device=self.device)
             ws = self._workspace(b)
             rc = self.lib.b200q_static_forward_u8(self.packed.ptr(), x_u8.data_ptr(), self.packed.input_lut.data_ptr(),
                                                   logits.data_ptr(), b, ws.data_ptr(), ws.numel(),

@@ -132,7 +132,9 @@ int b200q_quantize_conv3x3_first(const float* x, uint8_t* y, int64_t b, float in
  * then QuantStub): raw uint8 NHWC pixels [b,32,32,3] -> conv1 output uint8 NHWC [b,32,32,64].  lut_host is a HOST
  * table uint8[3][256], lut[c][v] = quantize_per_tensor(Normalize(ToTensor(v)))[c], built by the caller with the
  * reference's own torch ops (convnet_quantization_b200.packing.input_lut), so results are bit-identical to the fp32
- * route.  L must be conv1 (cin 4, cout 64, img 32) with host mirrors and B200Q_RQ_BOUNDED. */
+ * route.  L must be conv1 (cin 4, cout 64, img 32); x_nhwc 8-byte aligned, y 16-byte aligned.  Kernel selection is
+ * that of b200q_quantize_conv3x3_first (CUDA cores for a few images or for layers without host mirrors /
+ * B200Q_RQ_BOUNDED, tensor cores otherwise); results do not depend on it. */
 int b200q_u8_conv3x3_first(const uint8_t* x_nhwc, uint8_t* y, int64_t b, const uint8_t* lut_host,
                            const b200q_conv3x3* L, void* stream);
 #ifdef B200Q_DEV  /* development library (libb200q_dev.so) only: measured slower than the two kernels it replaces */
@@ -215,6 +217,13 @@ typedef struct b200q_graph b200q_graph;
  * default stream (CUDA cannot capture it); replays may go to any stream. */
 int b200q_graph_create(const b200q_static_net* net, const float* x_static, float* logits_static, int64_t b,
                        void* workspace, int64_t workspace_bytes, int flags, void* stream, b200q_graph** out);
+/* Same executor for the uint8 data path (b200q_static_forward_u8): x_nhwc_static is the caller's uint8 NHWC [b,32,32,3]
+ * pixel buffer.  lut_host (HOST uint8[3][256], see b200q_u8_conv3x3_first) is read during this call only: its contents
+ * are captured by value into kernel parameters, so the caller may free or change it afterwards (replays keep using the
+ * table as it was here).  Replay and destruction: b200q_graph_launch / b200q_graph_destroy. */
+int b200q_graph_create_u8(const b200q_static_net* net, const uint8_t* x_nhwc_static, const uint8_t* lut_host,
+                          float* logits_static, int64_t b, void* workspace, int64_t workspace_bytes, int flags,
+                          void* stream, b200q_graph** out);
 int b200q_graph_launch(b200q_graph* g, void* stream);
 int b200q_graph_destroy(b200q_graph* g);
 
