@@ -35,12 +35,14 @@ EXPORTS = (
     "b200q_linear_tc", "b200q_linear_simt", "b200q_linear_dequant", "b200q_linear_dynamic",
     "b200q_static_workspace_bytes", "b200q_static_forward", "b200q_static_forward_u8", "b200q_graph_create",
     "b200q_graph_create_u8", "b200q_graph_launch", "b200q_graph_destroy", "b200q_static_num_stages", "b200q_static_stage_name",
-    "b200q_static_forward_profiled",
+    "b200q_static_forward_profiled", "b200q_static_evaluate", "b200q_static_evaluate_u8",
 )
 DEV_EXPORTS = EXPORTS + ("b200q_conv12_fused", "b200q_conv3x3_simt")
 REDUCE_SCRATCH_BYTES = 8256    # B200Q_REDUCE_SCRATCH_BYTES
 REDUCE_QPARAMS_OFFSET = 8224   # B200Q_REDUCE_QPARAMS_OFFSET
 GRAPH_PDL = 1                  # B200Q_GRAPH_PDL
+EVAL_COUNTERS = 5              # B200Q_EVAL_COUNTERS, in the order of B200Q_EVAL_TOP1 .. B200Q_EVAL_TOP5_TIED
+EVAL_COUNTER_NAMES = ("top1", "top5", "images", "top1_tied", "top5_tied")
 
 
 class B200QError(RuntimeError):
@@ -139,6 +141,8 @@ _SIGNATURES = {
     "b200q_quantize_conv3x3_first": [_P, _P, _L, _F, C.POINTER(Conv3x3), _P],
     "b200q_u8_conv3x3_first": [_P, _P, _L, _P, C.POINTER(Conv3x3), _P],
     "b200q_static_forward_u8": [C.POINTER(StaticNet), _P, _P, _P, _L, _P, _L, _P],
+    "b200q_static_evaluate": [C.POINTER(StaticNet), _P, _P, _L, _P, _P, _P, _P, _L, _P],
+    "b200q_static_evaluate_u8": [C.POINTER(StaticNet), _P, _P, _P, _L, _P, _P, _P, _P, _L, _P],
     "b200q_conv3x3_tc": [_P, _P, _L, C.POINTER(Conv3x3), _I, _P],
     "b200q_linear_tc": [_P, _P, _L, C.POINTER(Linear), _P],
     "b200q_linear_simt": [_P, _P, _L, C.POINTER(Linear), _P],

@@ -46,10 +46,23 @@ int conv3x3_halo_dispatch(const uint8_t* x, uint8_t* y, int64_t b, const b200q_c
 // conv_halo2.cu: conv2 + fused pool on CTA pairs (tcgen05.mma.cta_group::2); returns 1 when not covered
 int conv3x3_halo2_dispatch(const uint8_t* x, uint8_t* y, int64_t b, const b200q_conv3x3* L, bool pool, cudaStream_t s,
                            int* rc);
+// Accuracy counting in the classifier head (b200q_static_evaluate, rule in b200q.h): labels int64 [b]; counters uint64
+// [B200Q_EVAL_COUNTERS], accumulated into; pred int32 [b] or nullptr.  The head kernels also skip the logits store when
+// their logits pointer is nullptr.
+struct EvalArgs {
+  const int64_t* labels;
+  unsigned long long* counters;
+  int32_t* pred;
+};
 // simt.cu: fc1 + ReLU + fc2 + dequantize in one launch for small batches (ticket must be zero on entry; the kernel leaves
-// it zero); returns 1 when the shapes / batch are not covered
+// it zero); returns 1 when the shapes / batch are not covered.  eval != nullptr: counts as well (EvalArgs).
 int fc_head_small_dispatch(const uint8_t* x, uint8_t* h, float* logits, unsigned int* ticket, int64_t b,
-                           const b200q_linear* fc1, const b200q_linear* fc2, float out_scale, cudaStream_t s, int* rc);
+                           const b200q_linear* fc1, const b200q_linear* fc2, float out_scale, const EvalArgs* eval,
+                           cudaStream_t s, int* rc);
+// simt.cu: fc2 + dequantize + accuracy counting (the head of b200q_linear_dequant); logits may be nullptr.  Refuses
+// (B200Q_ERR_INVALID_ARG) an fc2 that is not k = 512, n = 10 or buffers that are not 16-byte aligned.
+int linear_head_eval(const uint8_t* x, float* logits, int64_t b, const b200q_linear* L, float out_scale,
+                     const EvalArgs& eval, cudaStream_t s);
 // conv_small.cu: CUDA-core kernel for a handful of images (one round trip per layer); returns 1 when not covered
 int conv3x3_tiny_dispatch(const uint8_t* x, uint8_t* y, int64_t b, const b200q_conv3x3* L, bool pool, cudaStream_t s,
                           int* rc);

@@ -84,10 +84,13 @@ struct PdlScope {  // sets the thread's PDL launch flag for the lifetime of the 
 // ticket_is_zero: the caller is capturing a graph and guarantees the head kernel's ticket word (last 1 KiB of the
 // workspace) already holds 0 (it was zeroed before the capture and every forward leaves it zero); otherwise it is
 // cleared here.
+// eval (production path only, no taps / events): the head kernel also counts (b200q_static_evaluate); logits may be
+// nullptr then.
 int forward_impl(const b200q_static_net* net, const float* x, float* logits, int64_t b, void* workspace,
                  int64_t workspace_bytes, uint8_t* const* taps, cudaEvent_t* ev, void* stream,
-                 const uint8_t* x_u8 = nullptr, const uint8_t* lut_host = nullptr, bool ticket_is_zero = false) {
-  B200Q_REQUIRE(net && (((x || x_u8) && logits && workspace) || b == 0), "static_forward: null pointer");
+                 const uint8_t* x_u8 = nullptr, const uint8_t* lut_host = nullptr, bool ticket_is_zero = false,
+                 const EvalArgs* eval = nullptr) {
+  B200Q_REQUIRE(net && (((x || x_u8) && (logits || eval) && workspace) || b == 0), "static_forward: null pointer");
   B200Q_REQUIRE(b >= 0, "static_forward: negative batch");
   if (b == 0) return 0;
   B200Q_REQUIRE(workspace_bytes >= b200q_static_workspace_bytes(b), "static_forward: workspace too small (%lld < %lld)",
@@ -138,11 +141,15 @@ int forward_impl(const b200q_static_net* net, const float* x, float* logits, int
 #ifdef B200Q_DEV
       if (g_stop_after && steps_done >= g_stop_after) return 0;
 #endif
-      if (fc_head_small_dispatch(B, A, logits, ticket, b, &net->fc1, &net->fc2, net->out_scale, s, &hrc) == 0) return hrc;
+      if (fc_head_small_dispatch(B, A, logits, ticket, b, &net->fc1, &net->fc2, net->out_scale, eval, s, &hrc) == 0)
+        return hrc;
     }
     STEP(b200q_linear_tc(B, A, b, &net->fc1, stream));
     MARK();
-    STEP(b200q_linear_dequant(A, logits, b, &net->fc2, net->out_scale, stream));
+    if (eval)
+      STEP(linear_head_eval(A, logits, b, &net->fc2, net->out_scale, *eval, s));
+    else
+      STEP(b200q_linear_dequant(A, logits, b, &net->fc2, net->out_scale, stream));
     MARK();
     return 0;
   }
@@ -187,6 +194,39 @@ extern "C" int b200q_static_forward_u8(const b200q_static_net* net, const uint8_
                                        void* stream) {
   B200Q_REQUIRE(lut_host != nullptr && (x_nhwc != nullptr || b == 0), "static_forward_u8: null pointer");
   return forward_impl(net, nullptr, logits, b, workspace, workspace_bytes, nullptr, nullptr, stream, x_nhwc, lut_host);
+}
+
+namespace {
+int check_evaluate(const b200q_static_net* net, const int64_t* labels, int64_t b, const uint64_t* counters,
+                   const int32_t* pred) {
+  B200Q_REQUIRE(labels != nullptr && counters != nullptr, "static_evaluate: null labels or counters");
+  B200Q_REQUIRE(b >= 0, "static_evaluate: negative batch");
+  B200Q_REQUIRE((uintptr_t)labels % 8 == 0 && (uintptr_t)counters % 8 == 0 && (uintptr_t)pred % 4 == 0,
+                "static_evaluate: misaligned labels, counters or pred");
+  B200Q_REQUIRE(net != nullptr, "static_evaluate: null net");
+  B200Q_REQUIRE(net->fc2.k == 512 && net->fc2.n == 10, "static_evaluate: the counting head needs fc2 k=512 n=10 (k=%d n=%d)",
+                net->fc2.k, net->fc2.n);
+  return 0;
+}
+}  // namespace
+
+extern "C" int b200q_static_evaluate(const b200q_static_net* net, const float* x, const int64_t* labels, int64_t b,
+                                     uint64_t* counters, int32_t* pred, float* logits, void* workspace,
+                                     int64_t workspace_bytes, void* stream) {
+  if (int rc = check_evaluate(net, labels, b, counters, pred)) return rc;
+  const EvalArgs eval{labels, reinterpret_cast<unsigned long long*>(counters), pred};
+  return forward_impl(net, x, logits, b, workspace, workspace_bytes, nullptr, nullptr, stream, nullptr, nullptr, false,
+                      &eval);
+}
+
+extern "C" int b200q_static_evaluate_u8(const b200q_static_net* net, const uint8_t* x_nhwc, const uint8_t* lut_host,
+                                        const int64_t* labels, int64_t b, uint64_t* counters, int32_t* pred,
+                                        float* logits, void* workspace, int64_t workspace_bytes, void* stream) {
+  if (int rc = check_evaluate(net, labels, b, counters, pred)) return rc;
+  B200Q_REQUIRE(lut_host != nullptr && (x_nhwc != nullptr || b == 0), "static_evaluate_u8: null pointer");
+  const EvalArgs eval{labels, reinterpret_cast<unsigned long long*>(counters), pred};
+  return forward_impl(net, nullptr, logits, b, workspace, workspace_bytes, nullptr, nullptr, stream, x_nhwc, lut_host,
+                      false, &eval);
 }
 
 // ---------------------------------------------------------------------------------------------------- executor

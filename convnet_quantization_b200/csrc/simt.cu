@@ -232,12 +232,58 @@ __global__ void __launch_bounds__(256) linear_simt_kernel(const LinearArgs a) {
   }
 }
 
+// ---- accuracy counting inside the head (EVAL instantiations; the rule is stated in b200q.h at B200Q_EVAL_COUNTERS).
+// Called by the whole warp once per image, lane n < N holding the uint8 output q[n] (other lanes: anything).  The
+// uint8 values are compared, not the logits: dequantisation is strictly monotone.  Every lane ends with the same
+// counts; lane 0's are added up per CTA by eval_flush.
+template <int N>
+__device__ __forceinline__ void eval_image(uint32_t q, int lane, int64_t img, const EvalArgs& ev, uint32_t (&cnt)[5]) {
+  static_assert(N >= 1 && N <= 32, "one class per lane");
+  constexpr unsigned kClasses = N == 32 ? 0xffffffffu : (1u << N) - 1u;
+  constexpr int K5 = N < 5 ? N : 5;
+  const int64_t label = __ldg(ev.labels + img);
+  const bool valid = label >= 0 && label < N;
+  const int l = valid ? (int)label : 0;
+  const uint32_t ql = __shfl_sync(0xffffffffu, q, l);
+  const unsigned gt = __ballot_sync(0xffffffffu, q > ql) & kClasses;
+  const unsigned eq = __ballot_sync(0xffffffffu, q == ql) & kClasses;
+  const int g = __popc(gt), e = __popc(eq) - 1;  // e excludes the label itself
+  const int rank = g + __popc(eq & ((1u << l) - 1u));
+  if (valid) {
+    cnt[B200Q_EVAL_TOP1] += rank < 1;
+    cnt[B200Q_EVAL_TOP5] += rank < K5;
+    cnt[B200Q_EVAL_TOP1_TIED] += g < 1 && 1 <= g + e;
+    cnt[B200Q_EVAL_TOP5_TIED] += g < K5 && K5 <= g + e;
+  }
+  cnt[B200Q_EVAL_IMAGES] += 1;
+  if (ev.pred != nullptr) {  // rank-0 class: the first index holding the maximum
+    const uint32_t qmax = __reduce_max_sync(0xffffffffu, lane < N ? q : 0u);
+    const unsigned at_max = __ballot_sync(0xffffffffu, q == qmax) & kClasses;
+    if (lane == 0) ev.pred[img] = __ffs(at_max) - 1;
+  }
+}
+
+// Block-wide sum of lane 0's counts, then one global atomicAdd per (non-zero) counter per CTA.  Integer adds: the
+// totals do not depend on the order.  Every thread of the block must call it.
+__device__ __forceinline__ void eval_flush(const uint32_t (&cnt)[5], const EvalArgs& ev) {
+  __shared__ unsigned long long s_cnt[B200Q_EVAL_COUNTERS];
+  if (threadIdx.x < B200Q_EVAL_COUNTERS) s_cnt[threadIdx.x] = 0ull;
+  __syncthreads();
+  if ((threadIdx.x & 31) == 0)
+#pragma unroll
+    for (int i = 0; i < B200Q_EVAL_COUNTERS; ++i)
+      if (cnt[i]) atomicAdd(&s_cnt[i], (unsigned long long)cnt[i]);
+  __syncthreads();
+  if (threadIdx.x < B200Q_EVAL_COUNTERS && s_cnt[threadIdx.x]) atomicAdd(ev.counters + threadIdx.x, s_cnt[threadIdx.x]);
+}
+
 // Narrow head (fc2: k = 512, n = 10) fused with aten::dequantize.  The generic tile kernel above pads n to 64 and ran
 // this 8 MB layer at 29 us; here a warp owns one image at a time: lane l reads bytes [16l, 16l+16) of the image's row
 // (one coalesced 512-byte load per image), holds the matching 16 bytes of all N weight rows in registers, and the N
 // dot products are completed with the warp-reduce instruction.  Lane n then requantises and dequantises output n.
-template <int N>
-__global__ void __launch_bounds__(256) linear_head_dequant_kernel(const LinearArgs a) {
+// EVAL: also counts (eval_image); the logits store is skipped when a.y is nullptr.
+template <int N, bool EVAL>
+__global__ void __launch_bounds__(256) linear_head_dequant_kernel(const LinearArgs a, const EvalArgs ev) {
   const int lane = threadIdx.x & 31;
   const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
   pdl_launch_dependents();
@@ -251,6 +297,7 @@ __global__ void __launch_bounds__(256) linear_head_dequant_kernel(const LinearAr
   pdl_wait();  // x is the previous kernel's output (weights and constants above are not)
   uint4 xv = make_uint4(0, 0, 0, 0);
   if (warp < a.b) xv = __ldg(reinterpret_cast<const uint4*>(a.x + (int64_t)warp * 512) + lane);
+  uint32_t cnt[5] = {0, 0, 0, 0, 0};
   for (int64_t img = warp; img < a.b; img += nwarps) {
     const uint4 x = xv;
     if (img + nwarps < a.b) xv = __ldg(reinterpret_cast<const uint4*>(a.x + (img + nwarps) * 512) + lane);  // prefetch
@@ -266,9 +313,13 @@ __global__ void __launch_bounds__(256) linear_head_dequant_kernel(const LinearAr
     }
     if (lane < N) {
       const uint32_t q = requant_u8(mine - corr, bdiv, mult, a.zp_out, lo);
-      reinterpret_cast<float*>(a.y)[img * N + lane] = __fmul_rn(__int2float_rn((int)q - a.zp_out), a.out_scale);
+      if (!EVAL || a.y != nullptr)
+        reinterpret_cast<float*>(a.y)[img * N + lane] = __fmul_rn(__int2float_rn((int)q - a.zp_out), a.out_scale);
+      if constexpr (EVAL) mine = (int)q;
     }
+    if constexpr (EVAL) eval_image<N>((uint32_t)mine, lane, img, ev, cnt);
   }
+  if constexpr (EVAL) eval_flush(cnt, ev);
 }
 
 // =========================================================================================================
@@ -305,7 +356,9 @@ struct FcSmallArgs {
   float out_scale;
 };
 
-__global__ void __launch_bounds__(256) fc_head_small_kernel(const FcSmallArgs a) {
+// EVAL: the last CTA's fc2 stage also counts (eval_image), and skips the logits store when a.logits is nullptr.
+template <bool EVAL>
+__global__ void __launch_bounds__(256) fc_head_small_kernel(const FcSmallArgs a, const EvalArgs ev) {
   constexpr int K = 4096, N1 = 512, N2 = 10, CH = 4, KV = K / 16 / 32;  // KV: 16-byte vectors per lane and row
   __shared__ uint4 s_w[CH][K / 16];
   __shared__ bool s_last;
@@ -360,6 +413,7 @@ __global__ void __launch_bounds__(256) fc_head_small_kernel(const FcSmallArgs a)
   const int nn = lane < N2 ? lane : 0;
   const int corr = __ldg(a.corr2 + nn);
   const float bdiv = __ldg(a.bdiv2 + nn), mult = __ldg(a.mult2 + nn);
+  uint32_t cnt[5] = {0, 0, 0, 0, 0};
   for (int img = warp; img < a.b; img += 8) {
     const uint4 x = __ldcg(reinterpret_cast<const uint4*>(a.h + (int64_t)img * N1) + lane);  // written by other SMs: L2
     int mine = 0;
@@ -374,22 +428,44 @@ __global__ void __launch_bounds__(256) fc_head_small_kernel(const FcSmallArgs a)
     }
     if (lane < N2) {
       const uint32_t q = requant_u8(mine - corr, bdiv, mult, a.zp2, a.lo2);
-      a.logits[img * N2 + lane] = __fmul_rn(__int2float_rn((int)q - a.zp2), a.out_scale);
+      if (!EVAL || a.logits != nullptr) a.logits[img * N2 + lane] = __fmul_rn(__int2float_rn((int)q - a.zp2), a.out_scale);
+      if constexpr (EVAL) mine = (int)q;
     }
+    if constexpr (EVAL) eval_image<N2>((uint32_t)mine, lane, img, ev, cnt);
   }
+  if constexpr (EVAL) eval_flush(cnt, ev);
   if (tid == 0) *a.ticket = 0u;  // ready for the next forward on this workspace
 }
 
 // Returns 1 when the pair of layers / the batch is not the shape this kernel is written for.
 int fc_head_small_dispatch(const uint8_t* x, uint8_t* h, float* logits, unsigned int* ticket, int64_t b,
-                           const b200q_linear* fc1, const b200q_linear* fc2, float out_scale, cudaStream_t s, int* rc) {
+                           const b200q_linear* fc1, const b200q_linear* fc2, float out_scale, const EvalArgs* eval,
+                           cudaStream_t s, int* rc) {
   if (b < 1 || b > FC_SMALL_MAX_B || fc1->k != 4096 || fc1->n != 512 || fc2->k != 512 || fc2->n != 10) return 1;
   if ((uintptr_t)x % 16 || (uintptr_t)h % 16 || (uintptr_t)fc1->w % 16 || (uintptr_t)fc2->w % 16 || (uintptr_t)ticket % 4) return 1;
   FcSmallArgs a{x, h, logits, ticket, fc1->w, fc1->corr, fc1->rq.mult, fc1->rq.bdiv, fc2->w, fc2->corr, fc2->rq.mult,
                 fc2->rq.bdiv, (int)b, fc1->rq.zp_out, fc1->rq.relu ? fc1->rq.zp_out : 0, fc2->rq.zp_out,
                 fc2->rq.relu ? fc2->rq.zp_out : 0, out_scale};
-  *rc = launch_kernel("fc_head_small_kernel", fc_head_small_kernel, 512 / 4, 256, 0, s, a);
+  *rc = eval ? launch_kernel("fc_head_small_kernel", fc_head_small_kernel<true>, 512 / 4, 256, 0, s, a, *eval)
+             : launch_kernel("fc_head_small_kernel", fc_head_small_kernel<false>, 512 / 4, 256, 0, s, a, EvalArgs{});
   return 0;
+}
+
+// Warps of the head kernel for b images: <= 8 blocks of 8 warps per SM.
+static int head_blocks(int64_t b) {
+  const int64_t warps = b < (int64_t)num_sms() * 64 ? b : (int64_t)num_sms() * 64;
+  return (int)((warps + 7) / 8);
+}
+
+int linear_head_eval(const uint8_t* x, float* logits, int64_t b, const b200q_linear* L, float out_scale,
+                     const EvalArgs& eval, cudaStream_t s) {
+  B200Q_REQUIRE(L->k == 512 && L->n == 10 && (uintptr_t)x % 16 == 0 && (uintptr_t)L->w % 16 == 0,
+                "static_evaluate: the counting head needs fc2 k=512 n=10 and 16-byte aligned rows (k=%d n=%d)", L->k,
+                L->n);
+  if (b == 0) return 0;
+  LinearArgs a{x, logits, L->w, L->corr, L->rq.mult, L->rq.bdiv, b, L->k, L->n, L->rq.zp_out, L->rq.relu, out_scale};
+  return launch_kernel("linear_head_dequant_kernel", linear_head_dequant_kernel<10, true>, head_blocks(b), 256, 0, s, a,
+                       eval);
 }
 
 template <int EPI>
@@ -546,10 +622,8 @@ extern "C" int b200q_linear_dequant(const uint8_t* x, float* y, int64_t b, const
   if (b == 0) return 0;
   LinearArgs a{x, y, L->w, L->corr, L->rq.mult, L->rq.bdiv, b, L->k, L->n, L->rq.zp_out, L->rq.relu,
                out_scale};
-  if (L->k == 512 && L->n == 10 && (uintptr_t)x % 16 == 0 && (uintptr_t)L->w % 16 == 0) {
-    const int64_t warps = b < (int64_t)num_sms() * 64 ? b : (int64_t)num_sms() * 64;  // <= 8 blocks of 8 warps per SM
-    return launch_kernel("linear_head_dequant_kernel", linear_head_dequant_kernel<10>, (int)((warps + 7) / 8), 256, 0,
-                         (cudaStream_t)stream, a);
-  }
+  if (L->k == 512 && L->n == 10 && (uintptr_t)x % 16 == 0 && (uintptr_t)L->w % 16 == 0)
+    return launch_kernel("linear_head_dequant_kernel", linear_head_dequant_kernel<10, false>, head_blocks(b), 256, 0,
+                         (cudaStream_t)stream, a, EvalArgs{});
   return launch_linear<EPI_REQUANT_DEQUANT_F32>(a, (cudaStream_t)stream);
 }

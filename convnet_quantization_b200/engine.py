@@ -30,6 +30,15 @@ def _current_stream_handle(device_index: int) -> int:
     return torch.cuda.current_stream(device_index).cuda_stream
 
 
+def eval_result(counters: torch.Tensor) -> dict:
+    """The five counters of ``StaticEngine.evaluate`` as ints by name, plus ``top1_pct`` / ``top5_pct`` (of
+    ``images``).  Copies to the host (synchronises)."""
+    r = dict(zip(_lib.EVAL_COUNTER_NAMES, (int(v) for v in counters.tolist())))
+    r["top1_pct"] = 100.0 * r["top1"] / max(r["images"], 1)
+    r["top5_pct"] = 100.0 * r["top5"] / max(r["images"], 1)
+    return r
+
+
 class _Graph:
     """One captured forward (``b200q_graph_*``): fixed batch, fixed input / logits buffers, private workspace.
     ``u8``: ``x`` holds uint8 NHWC pixels (``b200q_graph_create_u8``), else fp32 NCHW images."""
@@ -226,6 +235,62 @@ class StaticEngine:
                                                   torch.cuda.current_stream().cuda_stream)
             _lib.check(rc, "static_forward_u8")
         return logits
+
+    def _check_eval_args(self, b: int, labels, counters, pred):
+        def bad(t, dtype, shape):
+            return (not torch.is_tensor(t) or not t.is_cuda or t.device != self.device or t.dtype != dtype
+                    or tuple(t.shape) != shape or not t.is_contiguous())
+        for name, t, dtype, shape in (("counters", counters, torch.int64, (_lib.EVAL_COUNTERS,)),
+                                      ("pred", pred, torch.int32, (b,)),
+                                      ("labels", labels, torch.int64, (b,))):
+            if (t is not None or name == "labels") and bad(t, dtype, shape):
+                got = f"{t.dtype} {tuple(t.shape)} on {t.device}" if torch.is_tensor(t) else type(t).__name__
+                raise _lib.B200QError(f"{name} must be a contiguous {dtype} {list(shape)} tensor on {self.device}, "
+                                      f"got {got}")
+
+    @torch.no_grad()
+    def _evaluate(self, x, labels, counters, pred, logits, u8: bool) -> torch.Tensor:
+        b = x.shape[0]
+        self._check_eval_args(b, labels, counters, pred)
+        self._check_out(logits, b)
+        ctx = _NULL_CTX if torch.cuda.current_device() == self.device.index else torch.cuda.device(self.device)
+        with ctx:
+            if counters is None:
+                counters = torch.zeros(_lib.EVAL_COUNTERS, dtype=torch.int64, device=self.device)
+            if b == 0:
+                return counters
+            ws = self._workspace(b)
+            ptr = lambda t: None if t is None else t.data_ptr()  # noqa: E731
+            stream = torch.cuda.current_stream().cuda_stream
+            if u8:
+                rc = self.lib.b200q_static_evaluate_u8(self.packed.ptr(), x.data_ptr(), self.packed.input_lut.data_ptr(),
+                                                       labels.data_ptr(), b, counters.data_ptr(), ptr(pred), ptr(logits),
+                                                       ws.data_ptr(), ws.numel(), stream)
+            else:
+                rc = self.lib.b200q_static_evaluate(self.packed.ptr(), x.data_ptr(), labels.data_ptr(), b,
+                                                    counters.data_ptr(), ptr(pred), ptr(logits), ws.data_ptr(),
+                                                    ws.numel(), stream)
+            _lib.check(rc, "static_evaluate_u8" if u8 else "static_evaluate")
+        return counters
+
+    def evaluate(self, x: torch.Tensor, labels: torch.Tensor, counters: torch.Tensor | None = None,
+                 pred: torch.Tensor | None = None, logits: torch.Tensor | None = None) -> torch.Tensor:
+        """Top-1 / top-5 counting inside the classifier head (``b200q_static_evaluate``; the tie rule is in
+        ``include/b200q.h``).  ``x``: fp32 NCHW ``[B,3,32,32]``, ``labels``: int64 ``[B]``, both on this device.
+        Returns the int64 ``[5]`` counters ``_lib.EVAL_COUNTER_NAMES`` - ``counters`` when given (ACCUMULATED into),
+        else a fresh zeroed tensor.  Optional outputs: ``pred`` int32 ``[B]`` (rank-0 class) and ``logits`` fp32
+        ``[B,10]`` (what ``forward`` returns).  Runs eagerly on the current stream (no CUDA graph) and never
+        synchronises: read the counters when the stream has got there."""
+        x = x.contiguous()
+        self._check_input(x, (3, 32, 32), torch.float32, "StaticEngine.evaluate")
+        return self._evaluate(x, labels, counters, pred, logits, u8=False)
+
+    def evaluate_u8(self, x_u8: torch.Tensor, labels: torch.Tensor, counters: torch.Tensor | None = None,
+                    pred: torch.Tensor | None = None, logits: torch.Tensor | None = None) -> torch.Tensor:
+        """``evaluate`` from raw pixels, uint8 NHWC ``[B,32,32,3]`` (the input of ``forward_u8``)."""
+        x_u8 = x_u8.contiguous()
+        self._check_input(x_u8, (32, 32, 3), torch.uint8, "StaticEngine.evaluate_u8")
+        return self._evaluate(x_u8, labels, counters, pred, logits, u8=True)
 
     def stage_names(self):
         return [self.lib.b200q_static_stage_name(i).decode() for i in range(self.lib.b200q_static_num_stages())]

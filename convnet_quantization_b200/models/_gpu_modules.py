@@ -20,7 +20,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from .. import _lib, ops
-from ..engine import StaticEngine
+from ..engine import StaticEngine, eval_result
 
 
 def _default_device() -> torch.device:
@@ -143,7 +143,10 @@ class _HostPipelined(_GpuResident):
             n = min(2 * n, cap)
         yield lo, b - lo
 
-    def _forward_host(self, x: torch.Tensor, u8: bool = False) -> torch.Tensor:
+    def _pipelined(self, x: torch.Tensor, u8: bool, run_chunk) -> None:
+        """Host ``x`` through the two-stream chunk plan: copies each chunk into its stream's staging buffer and calls
+        ``run_chunk(xin, k, lo, n)`` on that stream (``k``: stream index; ``[lo, lo+n)``: the chunk's images).  Returns
+        once both streams have finished."""
         b = x.shape[0]
         x = x.contiguous()
         pipe = self._pipeline()
@@ -151,9 +154,6 @@ class _HostPipelined(_GpuResident):
         if u8 and pipe["xu8"] is None:
             pipe["xu8"] = [torch.empty((chunk, 32, 32, 3), dtype=torch.uint8, device=self.engine_device) for _ in range(2)]
             pipe["yu8"] = [torch.empty((chunk, 10), dtype=torch.float32, device=self.engine_device) for _ in range(2)]
-        if pipe["out"] is None or pipe["out"].shape[0] < b:
-            pipe["out"] = torch.empty((max(b, self.HOST_CHUNK), 10), dtype=torch.float32).pin_memory()
-        out = pipe["out"][:b]
         cur = torch.cuda.current_stream(self.engine_device)
         for s in pipe["streams"]:
             s.wait_stream(cur)
@@ -161,12 +161,25 @@ class _HostPipelined(_GpuResident):
         for i, (lo, n) in enumerate(plan):
             k = i & 1
             with torch.cuda.stream(pipe["streams"][k]):  # per-stream buffers: reuse is ordered by the stream itself
-                xin, yout = (pipe["xu8"] if u8 else pipe["x"])[k][:n], (pipe["yu8"] if u8 else pipe["y"])[k][:n]
+                xin = (pipe["xu8"] if u8 else pipe["x"])[k][:n]
                 xin.copy_(x[lo:lo + n], non_blocking=True)
-                self._chunk_forward(xin, yout, u8)
-                out[lo:lo + n].copy_(yout, non_blocking=True)
+                run_chunk(xin, k, lo, n)
         for s in pipe["streams"]:
             s.synchronize()
+
+    def _forward_host(self, x: torch.Tensor, u8: bool = False) -> torch.Tensor:
+        b = x.shape[0]
+        pipe = self._pipeline()
+        if pipe["out"] is None or pipe["out"].shape[0] < b:
+            pipe["out"] = torch.empty((max(b, self.HOST_CHUNK), 10), dtype=torch.float32).pin_memory()
+        out = pipe["out"][:b]
+
+        def run_chunk(xin, k, lo, n):
+            yout = (pipe["yu8"] if u8 else pipe["y"])[k][:n]
+            self._chunk_forward(xin, yout, u8)
+            out[lo:lo + n].copy_(yout, non_blocking=True)
+
+        self._pipelined(x, u8, run_chunk)
         return out.clone()  # the pinned staging buffer is reused by the next call
 
 
@@ -217,6 +230,41 @@ class B200StaticQuantizedNet(_HostPipelined):
         if self.sync_on_forward:
             torch.cuda.current_stream(self.engine_device).synchronize()
         return y
+
+    @torch.no_grad()
+    def eval_counters(self, images: torch.Tensor, labels: torch.Tensor, u8: bool = False) -> torch.Tensor:
+        """int64 ``[5]`` counters (``_lib.EVAL_COUNTER_NAMES``) on the engine's device, not synchronised: ``evaluate``
+        without the read-back, for callers that reduce them further (``sharding.evaluate_sharded``).  Host images go
+        through the chunk pipeline of ``forward`` / ``forward_uint8``; the labels are copied to the device once."""
+        shape, dtype = ((32, 32, 3), torch.uint8) if u8 else ((3, 32, 32), torch.float32)
+        if images.dim() != 4 or tuple(images.shape[1:]) != shape or (u8 and images.dtype != torch.uint8):
+            raise _lib.B200QError(f"evaluate{'_uint8' if u8 else ''} expects {dtype} [B,{','.join(map(str, shape))}], "
+                                  f"got {images.dtype} {tuple(images.shape)}")
+        if labels.dtype != torch.int64 or tuple(labels.shape) != (images.shape[0],):
+            raise _lib.B200QError(f"labels must be int64 [{images.shape[0]}], got {labels.dtype} {tuple(labels.shape)}")
+        dev = self.engine_device
+        with torch.cuda.device(dev):
+            counters = torch.zeros(_lib.EVAL_COUNTERS, dtype=torch.int64, device=dev)
+            labels = labels.to(dev).contiguous()
+            run = self.engine.evaluate_u8 if u8 else self.engine.evaluate
+            if images.is_cuda:
+                run(images.to(dev, dtype), labels, counters)
+            elif images.shape[0] > 0:  # integer counts: chunking and the two streams change no total
+                self._pipelined(images.to(dtype), u8, lambda xin, k, lo, n: run(xin, labels[lo:lo + n], counters))
+        return counters
+
+    @torch.no_grad()
+    def evaluate(self, images: torch.Tensor, labels: torch.Tensor) -> dict:
+        """Top-1 / top-5 accuracy over fp32 NCHW ``images`` (CPU or CUDA) and int64 ``labels``, counted inside the
+        classifier-head kernel (tie rule: ``include/b200q.h``): ``{"top1", "top5", "images", "top1_tied",
+        "top5_tied", "top1_pct", "top5_pct"}``.  The ``*_tied`` counts bound how far a ``topk``-based count of the
+        same logits can differ.  Only the 40 bytes of counters come back to the host."""
+        return eval_result(self.eval_counters(images, labels))
+
+    @torch.no_grad()
+    def evaluate_uint8(self, pixels: torch.Tensor, labels: torch.Tensor) -> dict:
+        """``evaluate`` from raw uint8 NHWC pixels ``[B,32,32,3]`` (the input of ``forward_uint8``)."""
+        return eval_result(self.eval_counters(pixels, labels, u8=True))
 
     @torch.no_grad()
     def forward_with_taps(self, x):

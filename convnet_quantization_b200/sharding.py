@@ -2,9 +2,10 @@
 
 Static-PTQ and fp32 outputs are per-image independent, so rank ``r`` of ``R`` simply takes images
 ``[r*N/R, (r+1)*N/R)``; weights are replicated; there is no collective on the hot path.  The only exchange is one
-all-reduce of three int64 counters ``[top1, top5, total]`` at the end of a sweep (NCCL over NVLink on GPUs, gloo in the
-CPU tests).  The reference has no multi-process code at all; this mirrors what ``utils/model_evaluator.py:15-55``
-computes in one process.
+all-reduce of the int64 counters at the end of a sweep (NCCL over NVLink on GPUs, gloo in the CPU tests): three
+``[top1, top5, total]`` for ``sharded_accuracy`` (any model, ``topk`` counting), five for ``evaluate_sharded`` (the
+static-PTQ net's counting head, tie rule of ``include/b200q.h``).  The reference has no multi-process code at all;
+this mirrors what ``utils/model_evaluator.py:15-55`` computes in one process.
 """
 from __future__ import annotations
 
@@ -75,6 +76,30 @@ def topk_counts(logits: torch.Tensor, labels: torch.Tensor) -> torch.Tensor:
     return torch.stack([hit[:, 0].sum(), hit.sum(), torch.tensor(labels.numel(), device=logits.device)]).to(torch.int64)
 
 
+def rank_rule_hits(logits: torch.Tensor, labels: torch.Tensor) -> torch.Tensor:
+    """bool ``[B, 4]``: (top-1 hit, top-5 hit, top-1 tied, top-5 tied) per image under the counting rule of
+    ``b200q_static_evaluate`` (``include/b200q.h``), restated with torch ops on any device: hits follow the order of
+    ``torch.sort(logits, 1, descending=True, stable=True)``; "tied" means some order of the classes tied with the label
+    would flip the hit; a label outside ``[0, n)`` is a miss and not tied."""
+    n = logits.shape[1]
+    k5 = min(5, n)
+    valid = (labels >= 0) & (labels < n)
+    lab = torch.where(valid, labels, torch.zeros_like(labels)).view(-1, 1)
+    v = logits.gather(1, lab)
+    g = (logits > v).sum(1)
+    same = logits == v
+    e = same.sum(1) - 1
+    rank = g + (same & (torch.arange(n, device=logits.device).view(1, -1) < lab)).sum(1)
+    return torch.stack([valid & (rank < 1), valid & (rank < k5),
+                        valid & (g < 1) & (g + e >= 1), valid & (g < k5) & (g + e >= k5)], 1)
+
+
+def rank_rule_counts(logits: torch.Tensor, labels: torch.Tensor) -> torch.Tensor:
+    """int64 ``[top1, top5, images, top1_tied, top5_tied]`` of ``rank_rule_hits`` (the counters' layout)."""
+    h = rank_rule_hits(logits, labels).sum(0)
+    return torch.stack([h[0], h[1], torch.tensor(labels.numel(), device=logits.device), h[2], h[3]]).to(torch.int64)
+
+
 def allreduce_counts(counts: torch.Tensor) -> torch.Tensor:
     """Sum the per-rank counters over the default process group (no-op without one)."""
     if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
@@ -93,3 +118,13 @@ def sharded_accuracy(model, images: torch.Tensor, labels: torch.Tensor, rank: in
     counts = allreduce_counts(counts)
     t1, t5, n = (int(v) for v in counts.tolist())
     return 100.0 * t1 / max(n, 1), 100.0 * t5 / max(n, 1), n
+
+
+def evaluate_sharded(model, images: torch.Tensor, labels: torch.Tensor, rank: int, world: int, u8: bool = False) -> dict:
+    """This rank's shard through ``model.evaluate`` (``evaluate_uint8`` with ``u8``: uint8 NHWC pixels), then one
+    all-reduce of the five counters over the default process group (NCCL on GPUs).  Returns the global counts as
+    ``model.evaluate`` does; every rank gets the same result."""
+    from .engine import eval_result
+    lo, hi = shard_range(images.shape[0], rank, world)
+    counts = model.eval_counters(images[lo:hi], labels[lo:hi], u8=u8)
+    return eval_result(allreduce_counts(counts))

@@ -203,6 +203,36 @@ int b200q_static_forward(const b200q_static_net* net, const float* x, float* log
 int b200q_static_forward_u8(const b200q_static_net* net, const uint8_t* x_nhwc, const uint8_t* lut_host, float* logits,
                             int64_t b, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ---- accuracy counting (utils/model_evaluator.py:15-55: top-1 / top-5 hits over a labelled dataset) ----------------
+ * The forward above with the counting done by the classifier-head kernel itself: no extra launch, and the logits need
+ * not leave the device.  The rule, for one image with uint8 fc2 outputs q[0..n) and label L (uint8 values compared:
+ * dequantisation is strictly monotone, so the logits give the same result):
+ *   g = #{j : q[j] > q[L]},  e = #{j != L : q[j] == q[L]},  rank = g + #{j < L : q[j] == q[L]}
+ *   top-k hit   <=> rank < k            (k = 1 and k = min(5, n); the order of torch.sort(descending, stable), for k = 1
+ *                                        torch.argmax: ties go to the lower class index)
+ *   top-k tied  <=> g < k <= g + e      (some order of the tied classes would flip this image's hit; so a topk-based
+ *                                        count of the same logits differs from this one by at most the tied count)
+ * A label outside [0, n) is a miss and not tied; it still counts in IMAGES.
+ * counters: uint64 [B200Q_EVAL_COUNTERS] on the device (8-byte aligned), ACCUMULATED into (zero it first); integer
+ * adds, so the totals are deterministic. */
+#define B200Q_EVAL_COUNTERS 5
+#define B200Q_EVAL_TOP1 0
+#define B200Q_EVAL_TOP5 1
+#define B200Q_EVAL_IMAGES 2
+#define B200Q_EVAL_TOP1_TIED 3
+#define B200Q_EVAL_TOP5_TIED 4
+/* x fp32 NCHW [b,3,32,32]; labels int64 [b] (8-byte aligned); pred (optional, NULL skips it) int32 [b] receives the
+ * rank-0 class; logits (optional, NULL skips the store) fp32 [b,10] receives what b200q_static_forward writes.  Same
+ * kernels, launch count and workspace as b200q_static_forward (eager only: no graph).  Null labels or counters,
+ * b < 0 and misaligned labels / counters / pred are refused before any CUDA call.  fc2 must be k = 512, n = 10. */
+int b200q_static_evaluate(const b200q_static_net* net, const float* x, const int64_t* labels, int64_t b,
+                          uint64_t* counters, int32_t* pred, float* logits, void* workspace, int64_t workspace_bytes,
+                          void* stream);
+/* The same from raw uint8 NHWC pixels [b,32,32,3] (lut_host: see b200q_u8_conv3x3_first). */
+int b200q_static_evaluate_u8(const b200q_static_net* net, const uint8_t* x_nhwc, const uint8_t* lut_host,
+                             const int64_t* labels, int64_t b, uint64_t* counters, int32_t* pred, float* logits,
+                             void* workspace, int64_t workspace_bytes, void* stream);
+
 /* ---- whole-network executor (SURVEY 8f rank 1) -----------------------------------------------------------------
  * The forward captured ONCE as a CUDA graph for a fixed batch and fixed buffers, with programmatic dependent launch
  * between the layer kernels (kernel N+1's prologue - weights into shared memory, TMEM allocation, pad initialisation -
