@@ -35,7 +35,8 @@ EXPORTS = (
     "b200q_linear_tc", "b200q_linear_simt", "b200q_linear_dequant", "b200q_linear_dynamic",
     "b200q_static_workspace_bytes", "b200q_static_forward", "b200q_static_forward_u8", "b200q_graph_create",
     "b200q_graph_create_u8", "b200q_graph_launch", "b200q_graph_destroy", "b200q_static_num_stages", "b200q_static_stage_name",
-    "b200q_static_forward_profiled", "b200q_static_evaluate", "b200q_static_evaluate_u8",
+    "b200q_static_forward_profiled", "b200q_static_evaluate", "b200q_static_evaluate_u8", "b200q_sandwich_forward",
+    "b200q_sandwich_graph_create",
 )
 DEV_EXPORTS = EXPORTS + ("b200q_conv12_fused", "b200q_conv3x3_simt")
 REDUCE_SCRATCH_BYTES = 8256    # B200Q_REDUCE_SCRATCH_BYTES
@@ -122,6 +123,11 @@ class StaticNet(C.Structure):
                 ("fc1", Linear), ("fc2", Linear), ("out_scale", C.c_float)]
 
 
+class SandwichNet(C.Structure):
+    _fields_ = [("in_inv_scale", C.c_float), ("conv", Conv3x3 * 6), ("fc1", Linear), ("lut_host", (C.c_uint8 * 256) * 6),
+                ("fc1_scale", C.c_float), ("fc2_w", C.c_void_p), ("fc2_b", C.c_void_p)]
+
+
 _P, _I, _L, _F = C.c_void_p, C.c_int, C.c_int64, C.c_float
 _SIGNATURES = {
     "b200q_quantize_nchw_to_nhwc": [_P, _P, _L, _I, _I, _I, _I, _F, _I, _P],
@@ -151,6 +157,8 @@ _SIGNATURES = {
     "b200q_static_forward": [C.POINTER(StaticNet), _P, _P, _L, _P, _L, C.POINTER(C.c_void_p), _P],
     "b200q_static_forward_profiled": [C.POINTER(StaticNet), _P, _P, _L, _P, _L, C.POINTER(C.c_float), _P],
     "b200q_static_num_stages": [],
+    "b200q_sandwich_forward": [C.POINTER(SandwichNet), _P, _P, _L, _P, _L, C.POINTER(C.c_void_p), _P],
+    "b200q_sandwich_graph_create": [C.POINTER(SandwichNet), _P, _P, _L, _P, _L, _I, _P, C.POINTER(C.c_void_p)],
 }
 
 _DEV_SIGNATURES = {

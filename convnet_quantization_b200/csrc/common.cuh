@@ -63,6 +63,15 @@ int fc_head_small_dispatch(const uint8_t* x, uint8_t* h, float* logits, unsigned
 // (B200Q_ERR_INVALID_ARG) an fc2 that is not k = 512, n = 10 or buffers that are not 16-byte aligned.
 int linear_head_eval(const uint8_t* x, float* logits, int64_t b, const b200q_linear* L, float out_scale,
                      const EvalArgs& eval, cudaStream_t s);
+// simt.cu: the sandwich net's fp32 head (b200q_sandwich_forward; arithmetic stated in b200q.h).  fc1's uint8 output x
+// [b][512] (zero-point zp, DeQuantStub scale fc1_scale) -> logits [b][10]; fc2_w fp32 [10][512] 16-byte aligned, x too.
+int sandwich_head(const uint8_t* x, float* logits, int64_t b, const float* fc2_w, const float* fc2_b, int zp,
+                  float fc1_scale, cudaStream_t s);
+// ... and the same head fused with fc1 for b <= 32 (fc_head_small_kernel; ticket as for fc_head_small_dispatch);
+// returns 1 when the shapes / batch are not covered.
+int sandwich_head_small_dispatch(const uint8_t* x, uint8_t* h, float* logits, unsigned int* ticket, int64_t b,
+                                 const b200q_linear* fc1, const float* fc2_w, const float* fc2_b, float fc1_scale,
+                                 cudaStream_t s, int* rc);
 // conv_small.cu: CUDA-core kernel for a handful of images (one round trip per layer); returns 1 when not covered
 int conv3x3_tiny_dispatch(const uint8_t* x, uint8_t* y, int64_t b, const b200q_conv3x3* L, bool pool, cudaStream_t s,
                           int* rc);

@@ -334,14 +334,18 @@ __global__ void __launch_bounds__(256) histc_kernel(const float* __restrict__ x,
 // Byte-wise table look-up y[i] = lut[x[i]]: the table lives in shared memory replicated 32 times with a 4-byte
 // interleave (entry v of copy l at word v*32 + l), so the 32 lanes of a warp always hit 32 different banks whatever
 // bytes they look up.  16 bytes per thread and iteration.
+// In the sandwich forward's PDL chain (b200q_sandwich_forward) the table is filled while the previous conv still runs;
+// every access to x and y waits: x is that conv's output and y the buffer it reads.
 struct LutTable {
   uint8_t v[256];
 };
 __global__ void __launch_bounds__(256) lut_u8_kernel(const uint8_t* __restrict__ x, uint8_t* __restrict__ y, int64_t n,
                                                      const __grid_constant__ LutTable lut) {
   __shared__ uint32_t s_lut[256 * 32];
+  pdl_launch_dependents();
   for (int i = threadIdx.x; i < 256 * 32; i += blockDim.x) s_lut[i] = lut.v[i >> 5];
   __syncthreads();
+  pdl_wait();
   const uint32_t* tab = s_lut + (threadIdx.x & 31);
   auto map4 = [&](uint32_t w) {
     return tab[(w & 0xffu) << 5] | (tab[((w >> 8) & 0xffu) << 5] << 8) | (tab[((w >> 16) & 0xffu) << 5] << 16) |
@@ -451,6 +455,6 @@ extern "C" int b200q_lut_u8(const uint8_t* x, uint8_t* y, int64_t n, const uint8
   if (n == 0) return 0;
   LutTable t;
   for (int i = 0; i < 256; ++i) t.v[i] = lut_host[i];
-  lut_u8_kernel<<<grid_for(n / 16 + 1, 256, 4), 256, 0, (cudaStream_t)stream>>>(x, y, n, t);
-  return launched("lut_u8_kernel");
+  return launch_kernel("lut_u8_kernel", lut_u8_kernel, grid_for(n / 16 + 1, 256, 4), 256, 0, (cudaStream_t)stream, x, y,
+                       n, t);
 }

@@ -229,6 +229,105 @@ extern "C" int b200q_static_evaluate_u8(const b200q_static_net* net, const uint8
                       false, &eval);
 }
 
+// ---------------------------------------------------------------------------------------------------- sandwich net
+namespace {
+int check_sandwich(const b200q_sandwich_net* net, const float* x, const float* logits, int64_t b, const void* workspace,
+                   int64_t workspace_bytes) {
+  B200Q_REQUIRE(net != nullptr, "sandwich_forward: null net");
+  B200Q_REQUIRE(b >= 0, "sandwich_forward: negative batch");
+  B200Q_REQUIRE((x && logits && workspace) || b == 0, "sandwich_forward: null pointer");
+  B200Q_REQUIRE(workspace_bytes >= b200q_static_workspace_bytes(b),
+                "sandwich_forward: workspace too small (%lld < %lld)", (long long)workspace_bytes,
+                (long long)b200q_static_workspace_bytes(b));
+  static const int kGeom[6][3] = {{4, 64, 32}, {64, 64, 32}, {64, 128, 16}, {128, 128, 16}, {128, 256, 8}, {256, 256, 8}};
+  for (int i = 0; i < 6; ++i) {
+    const b200q_conv3x3& c = net->conv[i];
+    B200Q_REQUIRE(c.cin == kGeom[i][0] && c.cout == kGeom[i][1] && c.img == kGeom[i][2],
+                  "sandwich_forward: conv%d geometry (cin %d, cout %d, img %d) is not the net's (%d, %d, %d)", i + 1,
+                  c.cin, c.cout, c.img, kGeom[i][0], kGeom[i][1], kGeom[i][2]);
+  }
+  B200Q_REQUIRE(net->fc1.k == 4096 && net->fc1.n == 512, "sandwich_forward: fc1 must be 4096 -> 512 (got %d -> %d)",
+                net->fc1.k, net->fc1.n);
+  B200Q_REQUIRE(net->fc2_w && net->fc2_b && (uintptr_t)net->fc2_w % 16 == 0 && (uintptr_t)net->fc2_b % 4 == 0,
+                "sandwich_forward: fc2 (fp32 [10][512] + [10]) needs non-null pointers, weights 16-byte aligned");
+  return 0;
+}
+
+// Same buffers as forward_impl: A / B ping-pong of b x 64 KiB, the head's ticket word after B.  Every table reads the
+// conv output and writes the buffer that conv read; taps != nullptr materialises the un-pooled conv outputs.
+int sandwich_impl(const b200q_sandwich_net* net, const float* x, float* logits, int64_t b, void* workspace,
+                  int64_t workspace_bytes, uint8_t* const* taps, void* stream, bool ticket_is_zero = false) {
+  if (int rc = check_sandwich(net, x, logits, b, workspace, workspace_bytes)) return rc;
+  if (b == 0) return 0;
+  cudaStream_t s = (cudaStream_t)stream;
+  uint8_t* A = reinterpret_cast<uint8_t*>(align_up((int64_t)(uintptr_t)workspace, 1024));
+  uint8_t* B = A + align_up(b * BYTES_PER_IMG, 1024);
+  const b200q_conv3x3* L = net->conv;
+  const int zp_h = net->fc1.rq.zp_out;
+  int rc;
+#define STEP(call) do { rc = (call); if (rc) return rc; } while (0)
+#define LUT(i, src, dst, bytes_per_img) STEP(b200q_lut_u8(src, dst, b * (bytes_per_img), net->lut_host[i], stream))
+
+  if (taps == nullptr) {
+    PdlScope pdl(!ticket_is_zero && eager_pdl());  // (a capture sets the flag itself, from its B200Q_GRAPH_PDL flag)
+    STEP(b200q_quantize_conv3x3_first(x, A, b, net->in_inv_scale, &L[0], stream));  // -> [b,32,32,64]
+    LUT(0, A, B, 65536);
+    STEP(b200q_conv3x3_tc(B, A, b, &L[1], 1, stream));  // -> [b,16,16,64]
+    LUT(1, A, B, 16384);
+    STEP(b200q_conv3x3_tc(B, A, b, &L[2], 0, stream));  // -> [b,16,16,128]
+    LUT(2, A, B, 32768);
+    STEP(b200q_conv3x3_tc(B, A, b, &L[3], 1, stream));  // -> [b,8,8,128]
+    LUT(3, A, B, 8192);
+    STEP(b200q_conv3x3_tc(B, A, b, &L[4], 0, stream));  // -> [b,8,8,256]
+    LUT(4, A, B, 16384);
+    STEP(b200q_conv3x3_tc(B, A, b, &L[5], 1, stream));  // -> [b,4,4,256]
+    LUT(5, A, B, 4096);
+    unsigned int* ticket = reinterpret_cast<unsigned int*>(B + align_up(b * BYTES_PER_IMG, 1024));
+    if (b <= 32 && !ticket_is_zero) B200Q_CUDA(cudaMemsetAsync(ticket, 0, sizeof(unsigned int), s));
+    int hrc = 0;  // small batches: fc1 and the head in one kernel
+    if (sandwich_head_small_dispatch(B, A, logits, ticket, b, &net->fc1, net->fc2_w, net->fc2_b, net->fc1_scale, s,
+                                     &hrc) == 0)
+      return hrc;
+    STEP(b200q_linear_tc(B, A, b, &net->fc1, stream));
+    STEP(sandwich_head(A, logits, b, net->fc2_w, net->fc2_b, zp_h, net->fc1_scale, s));
+    return 0;
+  }
+
+  STEP(b200q_quantize_conv3x3_first(x, A, b, net->in_inv_scale, &L[0], stream));
+  STEP(copy_tap(taps, 0, A, b * 65536, s));
+  LUT(0, A, B, 65536);
+  STEP(b200q_conv3x3_tc(B, A, b, &L[1], 0, stream));
+  STEP(copy_tap(taps, 1, A, b * 65536, s));
+  STEP(b200q_max_pool2x2_nhwc(A, B, b, 32, 32, 64, stream));
+  LUT(1, B, A, 16384);
+  STEP(b200q_conv3x3_tc(A, B, b, &L[2], 0, stream));
+  STEP(copy_tap(taps, 2, B, b * 32768, s));
+  LUT(2, B, A, 32768);
+  STEP(b200q_conv3x3_tc(A, B, b, &L[3], 0, stream));
+  STEP(copy_tap(taps, 3, B, b * 32768, s));
+  STEP(b200q_max_pool2x2_nhwc(B, A, b, 16, 16, 128, stream));
+  LUT(3, A, B, 8192);
+  STEP(b200q_conv3x3_tc(B, A, b, &L[4], 0, stream));
+  STEP(copy_tap(taps, 4, A, b * 16384, s));
+  LUT(4, A, B, 16384);
+  STEP(b200q_conv3x3_tc(B, A, b, &L[5], 0, stream));
+  STEP(copy_tap(taps, 5, A, b * 16384, s));
+  STEP(b200q_max_pool2x2_nhwc(A, B, b, 8, 8, 256, stream));
+  LUT(5, B, A, 4096);
+  STEP(b200q_linear_tc(A, B, b, &net->fc1, stream));
+  STEP(copy_tap(taps, 6, B, b * 512, s));
+  STEP(sandwich_head(B, logits, b, net->fc2_w, net->fc2_b, zp_h, net->fc1_scale, s));
+#undef LUT
+#undef STEP
+  return 0;
+}
+}  // namespace
+
+extern "C" int b200q_sandwich_forward(const b200q_sandwich_net* net, const float* x, float* logits, int64_t b,
+                                      void* workspace, int64_t workspace_bytes, uint8_t* const* taps, void* stream) {
+  return sandwich_impl(net, x, logits, b, workspace, workspace_bytes, taps, stream);
+}
+
 // ---------------------------------------------------------------------------------------------------- executor
 struct b200q_graph {
   cudaGraph_t graph = nullptr;
@@ -238,29 +337,23 @@ struct b200q_graph {
 };
 
 namespace {
-// One capture body for both input kinds: x (fp32 NCHW) or x_u8 + lut_host (uint8 NHWC pixels, HOST table).
-int graph_create_impl(const b200q_static_net* net, const float* x, const uint8_t* x_u8, const uint8_t* lut_host,
-                      float* logits_static, int64_t b, void* workspace, int64_t workspace_bytes, int flags, void* stream,
-                      b200q_graph** out) {
-  B200Q_REQUIRE(out != nullptr, "graph_create: null out");
-  *out = nullptr;
-  B200Q_REQUIRE(net && (x || (x_u8 && lut_host)) && logits_static && workspace && b > 0,
-                "graph_create: null pointer or empty batch");
-  B200Q_REQUIRE(stream != nullptr, "graph_create: the legacy default stream cannot be captured; pass a created stream");
+// One capture body for every forward: fwd(ticket_is_zero) enqueues the whole forward on `stream`.  An eager forward
+// first (per-device kernel attributes, lazy module loading and the tensor-map encoder are first-use work that does not
+// belong inside a capture; it also leaves the small-batch head's ticket word zero), then the capture with the
+// B200Q_GRAPH_PDL flag, counting the kernels one replay launches.
+template <class Fwd>
+int capture_graph(int flags, void* stream, int64_t b, b200q_graph** out, Fwd&& fwd) {
   cudaStream_t s = (cudaStream_t)stream;
-  // eager first: per-device kernel attributes, lazy module loading and the tensor-map encoder are first-use work that
-  // does not belong inside a capture
-  int rc = forward_impl(net, x, logits_static, b, workspace, workspace_bytes, nullptr, nullptr, stream, x_u8, lut_host);
+  int rc = fwd(false);
   if (rc) return rc;
-  B200Q_CUDA(cudaStreamSynchronize(s));  // (the eager forward above left the head kernel's ticket word zero)
+  B200Q_CUDA(cudaStreamSynchronize(s));
   B200Q_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
   pdl_set((flags & B200Q_GRAPH_PDL) != 0);
 #ifdef B200Q_DEV
   g_stop_after = (flags >> 8) & 15;  // development library: capture only the first k kernels (timing breakdown)
 #endif
   const uint64_t launches0 = b200q_launch_count();
-  rc = forward_impl(net, x, logits_static, b, workspace, workspace_bytes, nullptr, nullptr, stream, x_u8, lut_host,
-                    /*ticket_is_zero=*/true);
+  rc = fwd(/*ticket_is_zero=*/true);
   const int captured_kernels = (int)(b200q_launch_count() - launches0);
   pdl_set(false);
 #ifdef B200Q_DEV
@@ -291,6 +384,26 @@ int graph_create_impl(const b200q_static_net* net, const float* x, const uint8_t
   *out = g;
   return 0;
 }
+
+int check_graph_args(const void* net, bool inputs, const float* logits_static, const void* workspace, int64_t b,
+                     void* stream, b200q_graph** out) {
+  B200Q_REQUIRE(out != nullptr, "graph_create: null out");
+  *out = nullptr;
+  B200Q_REQUIRE(net && inputs && logits_static && workspace && b > 0, "graph_create: null pointer or empty batch");
+  B200Q_REQUIRE(stream != nullptr, "graph_create: the legacy default stream cannot be captured; pass a created stream");
+  return 0;
+}
+
+// Both input kinds of the static net: x (fp32 NCHW) or x_u8 + lut_host (uint8 NHWC pixels, HOST table).
+int graph_create_impl(const b200q_static_net* net, const float* x, const uint8_t* x_u8, const uint8_t* lut_host,
+                      float* logits_static, int64_t b, void* workspace, int64_t workspace_bytes, int flags, void* stream,
+                      b200q_graph** out) {
+  if (int rc = check_graph_args(net, x || (x_u8 && lut_host), logits_static, workspace, b, stream, out)) return rc;
+  return capture_graph(flags, stream, b, out, [&](bool ticket_is_zero) {
+    return forward_impl(net, x, logits_static, b, workspace, workspace_bytes, nullptr, nullptr, stream, x_u8, lut_host,
+                        ticket_is_zero);
+  });
+}
 }  // namespace
 
 extern "C" int b200q_graph_create(const b200q_static_net* net, const float* x_static, float* logits_static, int64_t b,
@@ -304,6 +417,16 @@ extern "C" int b200q_graph_create_u8(const b200q_static_net* net, const uint8_t*
                                      void* stream, b200q_graph** out) {
   return graph_create_impl(net, nullptr, x_nhwc_static, lut_host, logits_static, b, workspace, workspace_bytes, flags,
                            stream, out);
+}
+
+extern "C" int b200q_sandwich_graph_create(const b200q_sandwich_net* net, const float* x_static, float* logits_static,
+                                           int64_t b, void* workspace, int64_t workspace_bytes, int flags, void* stream,
+                                           b200q_graph** out) {
+  if (int rc = check_graph_args(net, x_static != nullptr, logits_static, workspace, b, stream, out)) return rc;
+  if (int rc = check_sandwich(net, x_static, logits_static, b, workspace, workspace_bytes)) return rc;
+  return capture_graph(flags, stream, b, out, [&](bool ticket_is_zero) {
+    return sandwich_impl(net, x_static, logits_static, b, workspace, workspace_bytes, nullptr, stream, ticket_is_zero);
+  });
 }
 
 extern "C" int b200q_graph_launch(b200q_graph* g, void* stream) {

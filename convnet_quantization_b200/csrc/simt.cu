@@ -323,6 +323,67 @@ __global__ void __launch_bounds__(256) linear_head_dequant_kernel(const LinearAr
 }
 
 // =========================================================================================================
+// fp32 head of the sandwich net (b200q_sandwich_forward; b200q.h states the order): fc1's uint8 output through ReLU and
+// DeQuantStub, then fp32 fc2 + bias.  Called by the whole warp for one image: lane l holds bytes [16l, 16l+16) of the
+// 512-byte row, w4(n, j) returns this lane's float4 w[n][16l+4j .. 16l+4j+3], bias_n is fc2's bias of output `lane`
+// (lanes >= 10: anything).  Returns y[lane] on lanes < 10.  Each multiply and add rounds on its own (no FMA) and the
+// butterfly leaves the same sum in every lane, so the logits depend on neither the batch nor the kernel that calls it.
+constexpr int SW_K = 512, SW_N = 10;
+
+template <class W4>
+__device__ __forceinline__ float sandwich_head_image(uint4 q, int lane, int zp, float scale, float bias_n, W4 w4) {
+  const uint32_t words[4] = {q.x, q.y, q.z, q.w};
+  float h[16];
+#pragma unroll
+  for (int i = 0; i < 16; ++i) {
+    const int v = (int)((words[i / 4] >> (8 * (i % 4))) & 0xffu);
+    h[i] = __fmul_rn(__int2float_rn(max(v, zp) - zp), scale);
+  }
+  float mine = 0.f;
+#pragma unroll
+  for (int n = 0; n < SW_N; ++n) {
+    float p = 0.f;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const float4 w = w4(n, j);
+      p = j == 0 ? __fmul_rn(h[0], w.x) : __fadd_rn(p, __fmul_rn(h[4 * j], w.x));
+      p = __fadd_rn(p, __fmul_rn(h[4 * j + 1], w.y));
+      p = __fadd_rn(p, __fmul_rn(h[4 * j + 2], w.z));
+      p = __fadd_rn(p, __fmul_rn(h[4 * j + 3], w.w));
+    }
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) p = __fadd_rn(p, __shfl_xor_sync(0xffffffffu, p, d));
+    if (lane == n) mine = p;
+  }
+  return __fadd_rn(mine, bias_n);
+}
+
+// Large batches: one warp per image as in linear_head_dequant_kernel.  The 20 KB of fp32 weights go to shared memory
+// before the PDL wait, as [n][j][lane] float4s so that the 32 lanes of a warp read 32 consecutive float4s.
+__global__ void __launch_bounds__(256) sandwich_head_kernel(const uint8_t* __restrict__ x, float* __restrict__ y,
+                                                            int64_t b, const float* __restrict__ w,
+                                                            const float* __restrict__ bias, int zp, float scale) {
+  __shared__ float4 s_w[SW_N * 4 * 32];
+  const int lane = threadIdx.x & 31;
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
+  pdl_launch_dependents();
+  for (int i = threadIdx.x; i < SW_N * SW_K / 4; i += blockDim.x)  // source float4 i = (n * 32 + l) * 4 + j
+    s_w[((i / 128) * 4 + i % 4) * 32 + (i / 4) % 32] = __ldg(reinterpret_cast<const float4*>(w) + i);
+  const float bias_n = lane < SW_N ? __ldg(bias + lane) : 0.f;
+  __syncthreads();
+  pdl_wait();  // x is the previous kernel's output
+  const auto w4 = [&](int n, int j) { return s_w[(n * 4 + j) * 32 + lane]; };
+  uint4 xv = make_uint4(0, 0, 0, 0);
+  if (warp < b) xv = __ldg(reinterpret_cast<const uint4*>(x + (int64_t)warp * SW_K) + lane);
+  for (int64_t img = warp; img < b; img += nwarps) {
+    const uint4 q = xv;
+    if (img + nwarps < b) xv = __ldg(reinterpret_cast<const uint4*>(x + (img + nwarps) * SW_K) + lane);  // prefetch
+    const float v = sandwich_head_image(q, lane, zp, scale, bias_n, w4);
+    if (lane < SW_N) y[img * SW_N + lane] = v;
+  }
+}
+
+// =========================================================================================================
 // Small-batch classifier head (whole-network executor, b <= FC_SMALL_MAX_B): fc1 (+ReLU) and fc2 + dequantize in ONE
 // launch.  At batch 1 the tensor-core fc1 kernel is a chain of 128 dependent-ish MMAs behind a 256 KB weight stream on
 // eight SMs, followed by a second launch for ten dot products; here all 2 MB of fc1 weights are read once, 16 KB per
@@ -355,10 +416,19 @@ struct FcSmallArgs {
   int zp2, lo2;
   float out_scale;
 };
+// fc_head_small_kernel<false, true> (sandwich net): fp32 fc2 [10][512] and bias [10], fc1's DeQuantStub scale (its
+// zero-point is FcSmallArgs::zp1).
+struct F32HeadArgs {
+  const float* w;
+  const float* bias;
+  float scale;
+};
 
 // EVAL: the last CTA's fc2 stage also counts (eval_image), and skips the logits store when a.logits is nullptr.
-template <bool EVAL>
-__global__ void __launch_bounds__(256) fc_head_small_kernel(const FcSmallArgs a, const EvalArgs ev) {
+// F32HEAD (sandwich net): the last CTA runs the fp32 head (sandwich_head_image) instead of the int8 fc2 + dequantize.
+template <bool EVAL, bool F32HEAD = false>
+__global__ void __launch_bounds__(256) fc_head_small_kernel(const FcSmallArgs a, const EvalArgs ev,
+                                                            const F32HeadArgs f) {
   constexpr int K = 4096, N1 = 512, N2 = 10, CH = 4, KV = K / 16 / 32;  // KV: 16-byte vectors per lane and row
   __shared__ uint4 s_w[CH][K / 16];
   __shared__ bool s_last;
@@ -368,8 +438,10 @@ __global__ void __launch_bounds__(256) fc_head_small_kernel(const FcSmallArgs a,
 #pragma unroll
   for (int c = 0; c < CH; ++c) s_w[c][tid] = __ldg(reinterpret_cast<const uint4*>(a.w1 + (int64_t)(c0 + c) * K) + tid);
   uint4 w2[N2];  // every CTA prefetches fc2's 5 KB (only the last one uses them): hides the load behind fc1
+  if constexpr (!F32HEAD) {
 #pragma unroll
-  for (int n = 0; n < N2; ++n) w2[n] = __ldg(reinterpret_cast<const uint4*>(a.w2 + n * N1) + lane);
+    for (int n = 0; n < N2; ++n) w2[n] = __ldg(reinterpret_cast<const uint4*>(a.w2 + n * N1) + lane);
+  }
   const int myc = c0 + (lane & 3);
   const int corr1 = __ldg(a.corr1 + myc);
   const float bdiv1 = __ldg(a.bdiv1 + myc), mult1 = __ldg(a.mult1 + myc);
@@ -410,6 +482,17 @@ __global__ void __launch_bounds__(256) fc_head_small_kernel(const FcSmallArgs a,
   __syncthreads();
   if (!s_last) return;
   __threadfence();
+  if constexpr (F32HEAD) {
+    const float bias_n = lane < N2 ? __ldg(f.bias + lane) : 0.f;
+    const auto w4 = [&](int n, int j) { return __ldg(reinterpret_cast<const float4*>(f.w) + (n * 32 + lane) * 4 + j); };
+    for (int img = warp; img < a.b; img += 8) {
+      const uint4 q = __ldcg(reinterpret_cast<const uint4*>(a.h + (int64_t)img * N1) + lane);  // written by other SMs: L2
+      const float v = sandwich_head_image(q, lane, a.zp1, f.scale, bias_n, w4);
+      if (lane < N2) a.logits[img * N2 + lane] = v;
+    }
+    if (tid == 0) *a.ticket = 0u;
+    return;
+  }
   const int nn = lane < N2 ? lane : 0;
   const int corr = __ldg(a.corr2 + nn);
   const float bdiv = __ldg(a.bdiv2 + nn), mult = __ldg(a.mult2 + nn);
@@ -446,8 +529,10 @@ int fc_head_small_dispatch(const uint8_t* x, uint8_t* h, float* logits, unsigned
   FcSmallArgs a{x, h, logits, ticket, fc1->w, fc1->corr, fc1->rq.mult, fc1->rq.bdiv, fc2->w, fc2->corr, fc2->rq.mult,
                 fc2->rq.bdiv, (int)b, fc1->rq.zp_out, fc1->rq.relu ? fc1->rq.zp_out : 0, fc2->rq.zp_out,
                 fc2->rq.relu ? fc2->rq.zp_out : 0, out_scale};
-  *rc = eval ? launch_kernel("fc_head_small_kernel", fc_head_small_kernel<true>, 512 / 4, 256, 0, s, a, *eval)
-             : launch_kernel("fc_head_small_kernel", fc_head_small_kernel<false>, 512 / 4, 256, 0, s, a, EvalArgs{});
+  *rc = eval ? launch_kernel("fc_head_small_kernel", fc_head_small_kernel<true>, 512 / 4, 256, 0, s, a, *eval,
+                            F32HeadArgs{})
+             : launch_kernel("fc_head_small_kernel", fc_head_small_kernel<false>, 512 / 4, 256, 0, s, a, EvalArgs{},
+                             F32HeadArgs{});
   return 0;
 }
 
@@ -455,6 +540,25 @@ int fc_head_small_dispatch(const uint8_t* x, uint8_t* h, float* logits, unsigned
 static int head_blocks(int64_t b) {
   const int64_t warps = b < (int64_t)num_sms() * 64 ? b : (int64_t)num_sms() * 64;
   return (int)((warps + 7) / 8);
+}
+
+int sandwich_head_small_dispatch(const uint8_t* x, uint8_t* h, float* logits, unsigned int* ticket, int64_t b,
+                                 const b200q_linear* fc1, const float* fc2_w, const float* fc2_b, float fc1_scale,
+                                 cudaStream_t s, int* rc) {
+  if (b < 1 || b > FC_SMALL_MAX_B || fc1->k != 4096 || fc1->n != 512) return 1;
+  if ((uintptr_t)x % 16 || (uintptr_t)h % 16 || (uintptr_t)fc1->w % 16 || (uintptr_t)ticket % 4) return 1;
+  FcSmallArgs a{x, h, logits, ticket, fc1->w, fc1->corr, fc1->rq.mult, fc1->rq.bdiv, nullptr, nullptr, nullptr, nullptr,
+                (int)b, fc1->rq.zp_out, fc1->rq.relu ? fc1->rq.zp_out : 0, 0, 0, 0.f};
+  *rc = launch_kernel("fc_head_small_kernel", fc_head_small_kernel<false, true>, 512 / 4, 256, 0, s, a, EvalArgs{},
+                      F32HeadArgs{fc2_w, fc2_b, fc1_scale});
+  return 0;
+}
+
+int sandwich_head(const uint8_t* x, float* logits, int64_t b, const float* fc2_w, const float* fc2_b, int zp,
+                  float fc1_scale, cudaStream_t s) {
+  if (b == 0) return 0;
+  return launch_kernel("sandwich_head_kernel", sandwich_head_kernel, head_blocks(b), 256, 0, s, x, logits, b, fc2_w,
+                       fc2_b, zp, fc1_scale);
 }
 
 int linear_head_eval(const uint8_t* x, float* logits, int64_t b, const b200q_linear* L, float out_scale,

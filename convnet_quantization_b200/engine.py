@@ -8,7 +8,7 @@ from collections import OrderedDict
 import torch
 
 from . import _lib
-from .packing import PackedStaticNet
+from .packing import PackedSandwichNet, PackedStaticNet
 
 TAP_NAMES = ("quant", "conv1", "conv2", "pool1", "conv3", "conv4", "pool2", "conv5", "conv6", "pool3", "fc1", "fc2")
 TAP_SHAPES = {  # per image, NHWC (quant is NHWC4: channel 3 is padding)
@@ -17,6 +17,8 @@ TAP_SHAPES = {  # per image, NHWC (quant is NHWC4: channel 3 is padding)
     "conv6": (8, 8, 256), "pool3": (4, 4, 256), "fc1": (512,), "fc2": (10,),
 }
 
+
+SANDWICH_TAP_NAMES = ("conv1", "conv2", "conv3", "conv4", "conv5", "conv6", "fc1")  # int8 layer outputs, before ReLU
 
 _NULL_CTX = contextlib.nullcontext()
 
@@ -40,7 +42,7 @@ def eval_result(counters: torch.Tensor) -> dict:
 
 
 class _Graph:
-    """One captured forward (``b200q_graph_*``): fixed batch, fixed input / logits buffers, private workspace.
+    """One captured forward (``b200q_*graph_create*``): fixed batch, fixed input / logits buffers, private workspace.
     ``u8``: ``x`` holds uint8 NHWC pixels (``b200q_graph_create_u8``), else fp32 NCHW images."""
 
     def __init__(self, engine, x: torch.Tensor, logits: torch.Tensor, pdl: bool, u8: bool = False):
@@ -54,14 +56,7 @@ class _Graph:
         side = engine._capture_stream()
         side.wait_stream(cur)
         flags = _lib.GRAPH_PDL if pdl else 0
-        if u8:
-            rc = lib.b200q_graph_create_u8(engine.packed.ptr(), x.data_ptr(), engine.packed.input_lut.data_ptr(),
-                                           logits.data_ptr(), b, self.ws.data_ptr(), self.ws.numel(), flags,
-                                           side.cuda_stream, C.byref(self.handle))
-        else:
-            rc = lib.b200q_graph_create(engine.packed.ptr(), x.data_ptr(), logits.data_ptr(), b, self.ws.data_ptr(),
-                                        self.ws.numel(), flags, side.cuda_stream, C.byref(self.handle))
-        _lib.check(rc, "graph_create_u8" if u8 else "graph_create")
+        engine._create_graph(x, logits, self.ws, flags, side.cuda_stream, C.byref(self.handle), u8)
         cur.wait_stream(side)
 
     def launch(self, stream: int):
@@ -76,35 +71,33 @@ class _Graph:
             pass
 
 
-class StaticEngine:
-    """Runs ``b200q_static_forward`` on one CUDA device.  fp32 NCHW ``[B,3,32,32]`` (CUDA) -> fp32 logits ``[B,10]``.
-
-    Whole-network executor (SURVEY 8f rank 1): batches of at most ``GRAPH_MAX_BATCH`` images - the latency-bound
-    regime the reference's own driver measures (``utils/inference_benchmark.py:126-138``: batch 1 and 32) - are
-    replayed from a CUDA graph captured on the caller's input buffer, with programmatic dependent launch between the
-    layer kernels.  A graph is captured the second time the same (batch, input buffer[, output buffer]) is seen and
-    ``GRAPH_CACHE`` of them are kept (least recently used evicted).  ``forward_u8`` (raw uint8 pixels) follows the
-    same policy; its graphs share the cache, keyed apart by the input kind."""
+class _NetEngine:
+    """What the whole-network engines share: eager workspaces (one per CUDA stream, LRU) and the whole-network executor
+    (SURVEY 8f rank 1).  Batches of at most ``GRAPH_MAX_BATCH`` images - the latency-bound regime the reference's own
+    driver measures (``utils/inference_benchmark.py:126-138``: batch 1 and 32) - are replayed from a CUDA graph
+    captured on the caller's input buffer, with programmatic dependent launch between the layer kernels.  A graph is
+    captured the second time the same (input kind, batch, input buffer[, output buffer]) is seen and ``GRAPH_CACHE`` of
+    them are kept (least recently used evicted).  Subclasses provide ``_create_graph``."""
 
     GRAPH_MAX_BATCH = 1024
     GRAPH_CACHE = 8
     WORKSPACE_CACHE = 4  # eager workspaces kept, one per CUDA stream that called forward (LRU)
 
-    def __init__(self, qparams: dict, device="cuda", use_graphs: bool = True, pdl: bool = True):
+    def __init__(self, device, use_graphs: bool, pdl: bool):
         self.device = torch.device(device)
         if self.device.type != "cuda":
-            raise _lib.B200QError("StaticEngine needs a CUDA device (no CPU fallback)")
+            raise _lib.B200QError(f"{type(self).__name__} needs a CUDA device (no CPU fallback)")
         if self.device.index is None:
             self.device = torch.device("cuda", torch.cuda.current_device())
         self.lib = _lib.load()
-        self.qparams = qparams
         self.use_graphs, self.pdl = use_graphs, pdl
-        with torch.cuda.device(self.device):
-            self.packed = PackedStaticNet(qparams, self.device)
         self._ws = OrderedDict()      # CUDA stream handle -> workspace (forwards on different streams must not share one)
         self._graphs = OrderedDict()  # (uint8 input?, batch, x ptr, out ptr or 0) -> _Graph
         self._seen = OrderedDict()    # keys seen once (capture on the second sighting)
         self._side = None
+
+    def _create_graph(self, x, logits, ws, flags: int, stream: int, handle_ref, u8: bool) -> None:
+        raise NotImplementedError
 
     def _capture_stream(self):
         if self._side is None:
@@ -165,6 +158,51 @@ class StaticEngine:
             self._graphs.popitem(last=False)
         return g
 
+    def _replay(self, x: torch.Tensor, out, graph, u8: bool = False):
+        """Logits from a graph replay on the current stream when the policy (or ``graph=True``) says so, else None."""
+        use_graph = self.use_graphs and x.shape[0] <= self.GRAPH_MAX_BATCH if graph is None else graph
+        if not use_graph:
+            return None
+        g = self._graph_for(x, out, u8)
+        if g is None and graph:  # forced: capture right away
+            g = self._graph_for(x, out, u8)
+        if g is None:
+            return None
+        g.launch(_current_stream_handle(self.device.index))
+        return out if out is not None else g.logits.clone()
+
+    def _tap_buffers(self, b: int, names, shapes):
+        """uint8 NHWC tap tensors by name and the C array of their pointers."""
+        arr = (C.c_void_p * len(names))()
+        tensors = {}
+        for i, name in enumerate(names):
+            t = torch.empty((b,) + shapes[name], dtype=torch.uint8, device=self.device)
+            tensors[name] = t
+            arr[i] = t.data_ptr()
+        return tensors, arr
+
+
+class StaticEngine(_NetEngine):
+    """Runs ``b200q_static_forward`` on one CUDA device.  fp32 NCHW ``[B,3,32,32]`` (CUDA) -> fp32 logits ``[B,10]``.
+    Small batches run on the whole-network executor (``_NetEngine``).  ``forward_u8`` (raw uint8 pixels) follows the
+    same policy; its graphs share the cache, keyed apart by the input kind."""
+
+    def __init__(self, qparams: dict, device="cuda", use_graphs: bool = True, pdl: bool = True):
+        super().__init__(device, use_graphs, pdl)
+        self.qparams = qparams
+        with torch.cuda.device(self.device):
+            self.packed = PackedStaticNet(qparams, self.device)
+
+    def _create_graph(self, x, logits, ws, flags, stream, handle_ref, u8):
+        if u8:
+            rc = self.lib.b200q_graph_create_u8(self.packed.ptr(), x.data_ptr(), self.packed.input_lut.data_ptr(),
+                                                logits.data_ptr(), x.shape[0], ws.data_ptr(), ws.numel(), flags, stream,
+                                                handle_ref)
+        else:
+            rc = self.lib.b200q_graph_create(self.packed.ptr(), x.data_ptr(), logits.data_ptr(), x.shape[0],
+                                             ws.data_ptr(), ws.numel(), flags, stream, handle_ref)
+        _lib.check(rc, "graph_create_u8" if u8 else "graph_create")
+
     @torch.no_grad()
     def forward(self, x: torch.Tensor, taps: bool = False, out: torch.Tensor | None = None, graph: bool | None = None):
         """``out`` (optional): preallocated fp32 ``[B,10]`` CUDA tensor to receive the logits.  ``graph``: force
@@ -182,25 +220,16 @@ class StaticEngine:
             if b == 0:
                 logits = out if out is not None else torch.empty((0, 10), dtype=torch.float32, device=self.device)
                 return (logits, {}) if taps else logits
-            use_graph = self.use_graphs and b <= self.GRAPH_MAX_BATCH if graph is None else graph
-            if use_graph and not taps:
-                g = self._graph_for(x, out)
-                if g is None and graph:  # forced: capture right away
-                    g = self._graph_for(x, out)
-                if g is not None:
-                    g.launch(_current_stream_handle(self.device.index))
-                    return out if out is not None else g.logits.clone()
+            if not taps:
+                y = self._replay(x, out, graph)
+                if y is not None:
+                    return y
             logits = out if out is not None else torch.empty((b, 10), dtype=torch.float32, device=self.device)
             ws = self._workspace(b)
             tap_ptrs = None
             tap_tensors = {}
             if taps:
-                arr = (C.c_void_p * len(TAP_NAMES))()
-                for i, name in enumerate(TAP_NAMES):
-                    t = torch.empty((b,) + TAP_SHAPES[name], dtype=torch.uint8, device=self.device)
-                    tap_tensors[name] = t
-                    arr[i] = t.data_ptr()
-                tap_ptrs = arr
+                tap_tensors, tap_ptrs = self._tap_buffers(b, TAP_NAMES, TAP_SHAPES)
             rc = self.lib.b200q_static_forward(self.packed.ptr(), x.data_ptr(), logits.data_ptr(), b, ws.data_ptr(),
                                                ws.numel(), tap_ptrs, torch.cuda.current_stream().cuda_stream)
             _lib.check(rc, "static_forward")
@@ -220,14 +249,9 @@ class StaticEngine:
         with ctx:
             if b == 0:
                 return out if out is not None else torch.empty((0, 10), dtype=torch.float32, device=self.device)
-            use_graph = self.use_graphs and b <= self.GRAPH_MAX_BATCH if graph is None else graph
-            if use_graph:
-                g = self._graph_for(x_u8, out, u8=True)
-                if g is None and graph:  # forced: capture right away
-                    g = self._graph_for(x_u8, out, u8=True)
-                if g is not None:
-                    g.launch(_current_stream_handle(self.device.index))
-                    return out if out is not None else g.logits.clone()
+            y = self._replay(x_u8, out, graph, u8=True)
+            if y is not None:
+                return y
             logits = out if out is not None else torch.empty((b, 10), dtype=torch.float32, device=self.device)
             ws = self._workspace(b)
             rc = self.lib.b200q_static_forward_u8(self.packed.ptr(), x_u8.data_ptr(), self.packed.input_lut.data_ptr(),
@@ -311,3 +335,50 @@ class StaticEngine:
                                                         torch.cuda.current_stream().cuda_stream)
             _lib.check(rc, "static_forward_profiled")
         return logits, dict(zip(self.stage_names(), (float(v) for v in ms)))
+
+
+class SandwichEngine(_NetEngine):
+    """Runs ``b200q_sandwich_forward`` (the per-layer sandwich net, ``ptq.calibrate_sandwich`` parameters) on one CUDA
+    device: fp32 NCHW ``[B,3,32,32]`` (CUDA) -> fp32 logits ``[B,10]``, with the executor policy of ``_NetEngine``.
+    The logits of an image do not depend on the batch it comes in, nor on eager / graph / PDL: the fp32 head has one
+    fixed summation order (``include/b200q.h``, restated in numpy by ``tests/test_gpu_sandwich_forward.py``)."""
+
+    def __init__(self, sparams: dict, device="cuda", use_graphs: bool = True, pdl: bool = True):
+        super().__init__(device, use_graphs, pdl)
+        self.sparams = sparams
+        with torch.cuda.device(self.device):
+            self.packed = PackedSandwichNet(sparams, self.device)
+
+    def _create_graph(self, x, logits, ws, flags, stream, handle_ref, u8):
+        rc = self.lib.b200q_sandwich_graph_create(self.packed.ptr(), x.data_ptr(), logits.data_ptr(), x.shape[0],
+                                                  ws.data_ptr(), ws.numel(), flags, stream, handle_ref)
+        _lib.check(rc, "sandwich_graph_create")
+
+    @torch.no_grad()
+    def forward(self, x: torch.Tensor, taps: bool = False, out: torch.Tensor | None = None, graph: bool | None = None):
+        """``taps``: also return ``{layer: uint8 NHWC output}`` of conv1..conv6 (un-pooled) and fc1 (``[B,512]``), the
+        int8 layers' outputs before ReLU.  ``out`` and ``graph`` as for ``StaticEngine.forward``."""
+        if x.is_cuda and x.dtype != torch.float32:
+            x = x.float()
+        x = x.contiguous()
+        self._check_input(x, (3, 32, 32), torch.float32, "SandwichEngine.forward")
+        b = x.shape[0]
+        self._check_out(out, b)
+        ctx = _NULL_CTX if torch.cuda.current_device() == self.device.index else torch.cuda.device(self.device)
+        with ctx:
+            if b == 0:
+                logits = out if out is not None else torch.empty((0, 10), dtype=torch.float32, device=self.device)
+                return (logits, {}) if taps else logits
+            if not taps:
+                y = self._replay(x, out, graph)
+                if y is not None:
+                    return y
+            logits = out if out is not None else torch.empty((b, 10), dtype=torch.float32, device=self.device)
+            ws = self._workspace(b)
+            tap_tensors, tap_ptrs = self._tap_buffers(b, SANDWICH_TAP_NAMES, TAP_SHAPES) if taps else ({}, None)
+            rc = self.lib.b200q_sandwich_forward(self.packed.ptr(), x.data_ptr(), logits.data_ptr(), b, ws.data_ptr(),
+                                                 ws.numel(), tap_ptrs, _current_stream_handle(self.device.index))
+            _lib.check(rc, "sandwich_forward")
+        return (logits, tap_tensors) if taps else logits
+
+    __call__ = forward

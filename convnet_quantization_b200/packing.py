@@ -171,3 +171,41 @@ class PackedStaticNet:
 
     def weight_bytes(self) -> int:
         return sum(p.w.numel() for p in self.convs) + self.fc1.w.numel() + self.fc2.w.numel()
+
+
+class PackedSandwichNet:
+    """Device constants of the per-layer sandwich net (``ptq.calibrate_sandwich``) + the ``b200q_sandwich_net`` struct.
+
+    conv1..conv6 and fc1 are packed as in the static net with ReLU fusion off and each layer's own QuantStub
+    (``in_scale`` / ``in_zp``); ``luts[i]`` is the boundary table (DeQuantStub -> ReLU -> next QuantStub) after layer i
+    (``ptq.sandwich_boundary_lut``); fc2 stays fp32."""
+
+    def __init__(self, sp: dict, device):
+        from . import ptq
+        self.device = torch.device(device)
+        names = ptq.SANDWICH_LAYERS
+        self.convs = [PackedConv(n, sp[n], sp[n]["in_scale"], sp[n]["in_zp"], self.device, relu=False) for n in names[:6]]
+        self.fc1 = PackedLinear("fc1", sp["fc1"], sp["fc1"]["in_scale"], sp["fc1"]["in_zp"], self.device, relu=False,
+                                nhwc_from=(256, 4, 4))
+        self.fc1_scale, self.fc1_zp = float(sp["fc1"]["out_scale"]), int(sp["fc1"]["out_zp"])
+        self.fc2_w = sp["fc2"]["weight"].detach().to(self.device, torch.float32).contiguous()
+        self.fc2_b = sp["fc2"]["bias"].detach().to(self.device, torch.float32).contiguous()
+        if tuple(self.fc2_w.shape) != (10, 512) or tuple(self.fc2_b.shape) != (10,):
+            raise _lib.B200QError(f"sandwich fc2 must be fp32 [10,512] + [10], got {tuple(self.fc2_w.shape)} + "
+                                  f"{tuple(self.fc2_b.shape)}")
+        self.luts = [ptq.sandwich_boundary_lut(sp[a]["out_scale"], sp[a]["out_zp"], sp[b]["in_scale"], sp[b]["in_zp"])
+                     for a, b in zip(names[:-1], names[1:])]
+        s_in = float(sp["conv1"]["in_scale"])
+        net = _lib.SandwichNet()
+        net.in_inv_scale = float(torch.tensor(1.0, dtype=torch.float32) / torch.tensor(s_in, dtype=torch.float32))
+        for i, pc in enumerate(self.convs):
+            net.conv[i] = pc.c
+        net.fc1 = self.fc1.c
+        for i, lut in enumerate(self.luts):
+            C.memmove(net.lut_host[i], lut.numpy().tobytes(), 256)
+        net.fc1_scale = self.fc1_scale
+        net.fc2_w, net.fc2_b = self.fc2_w.data_ptr(), self.fc2_b.data_ptr()
+        self.c = net
+
+    def ptr(self):
+        return C.byref(self.c)

@@ -257,6 +257,39 @@ int b200q_graph_create_u8(const b200q_static_net* net, const uint8_t* x_nhwc_sta
 int b200q_graph_launch(b200q_graph* g, void* stream);
 int b200q_graph_destroy(b200q_graph* g);
 
+/* ---- per-layer "sandwich" network (models/custom_quantization_model.py:34-58, 202-261) ------------------------------
+ * conv1..conv6 and fc1 each in QuantStub -> int8 layer -> DeQuantStub, fp32 ReLU / max-pool between them, fc2 in fp32.
+ * Between two int8 layers, DeQuantStub -> ReLU -> next QuantStub is the monotone uint8 -> uint8 table lut_host[i]
+ * (b200q_lut_u8); it commutes with the max-pool, so after conv2 / conv4 / conv6 it runs on the pooled tensor. */
+typedef struct b200q_sandwich_net {
+  float in_inv_scale;          /* 1.0f / conv1's QuantStub scale; its zero-point is conv[0].zp_x */
+  b200q_conv3x3 conv[6];       /* rq.relu == 0 (the sandwich's output observer sees pre-ReLU values) */
+  b200q_linear fc1;            /* rq.relu == 0; k 4096 in NHWC column order, n 512 */
+  uint8_t lut_host[6][256];    /* boundary tables conv1->conv2 ... conv5->conv6, conv6->fc1 (ptq.sandwich_boundary_lut) */
+  float fc1_scale;             /* fc1's DeQuantStub; zero-point fc1.rq.zp_out */
+  const float* fc2_w;          /* fp32 [10][512], device, 16-byte aligned */
+  const float* fc2_b;          /* fp32 [10], device, 4-byte aligned */
+} b200q_sandwich_net;
+
+/* fp32 NCHW [b,3,32,32] -> fp32 logits [b,10].  Workspace: b200q_static_workspace_bytes(b) (the same ping-pong buffers
+ * and ticket word as b200q_static_forward).  Enqueues 14 kernels (13 for b <= 32, where fc1 and the head are one
+ * kernel): quantize+conv1, then table + conv for conv2..conv6 (pools fused into conv2 / conv4 / conv6), the conv6->fc1
+ * table, fc1, and the fp32 head.  The head is defined to the bit, independently of the batch and of the kernel:
+ *   h[k] = f32(max(q[k], zp) - zp) * fc1_scale                       (ReLU + DeQuantStub of fc1's uint8 output q)
+ *   p[l] = (((h[16l]*w[16l]) + h[16l+1]*w[16l+1]) + ...) + h[16l+15]*w[16l+15]   for l = 0..31, one rounding per op
+ *   s    = butterfly: p[l] += p[l^16], then ^8, ^4, ^2, ^1 (every l ends with the same value)
+ *   y[n] = s + fc2_b[n]                                              (w = fc2_w[n], all fp32, no FMA)
+ * taps (optional, may be NULL): 7 device pointers receiving the uint8 NHWC output of conv1..conv6 (before ReLU and
+ * pooling) and fc1; that route runs the pools as kernels of their own.  A null net, b < 0, a short workspace, layer
+ * geometry other than the net's, fc1 other than 4096 -> 512, or null / misaligned fc2 pointers are refused with
+ * B200Q_ERR_INVALID_ARG before any CUDA call. */
+int b200q_sandwich_forward(const b200q_sandwich_net* net, const float* x, float* logits, int64_t b,
+                           void* workspace, int64_t workspace_bytes, uint8_t* const* taps, void* stream);
+/* Whole-network executor for b200q_sandwich_forward (as b200q_graph_create; replay and destruction:
+ * b200q_graph_launch / b200q_graph_destroy).  The six tables are read during this call only. */
+int b200q_sandwich_graph_create(const b200q_sandwich_net* net, const float* x_static, float* logits_static, int64_t b,
+                                void* workspace, int64_t workspace_bytes, int flags, void* stream, b200q_graph** out);
+
 /* Measurement hook (bench.py roofline): the same forward with a CUDA event recorded on `stream` before every layer
  * kernel and after the last one; synchronises on the last event and writes b200q_static_num_stages() per-kernel
  * durations in milliseconds to stage_ms_host (HOST memory).  Stage i is named b200q_static_stage_name(i). */
