@@ -243,6 +243,24 @@ __device__ __forceinline__ uint32_t requant4_prebiased(uint32_t v0, uint32_t v1,
   return pack_sat_u8(q1, q0, pack_sat_u8(q3, q2, 0u));
 }
 
+// Variant for fp32 accumulators that already hold f32(acc - corr) exactly (conv1_tc.cu: fp16 MMAs on x - zp, every
+// partial sum an integer below 2^20): fbgemm's arithmetic starts right at the bias add.  Valid when |t| < 2^22, which
+// B200Q_RQ_BOUNDED constants guarantee for |acc - corr| < 2^20.
+__device__ __forceinline__ uint32_t requant4_f32acc(uint32_t v0, uint32_t v1, uint32_t v2, uint32_t v3, const float4 bd,
+                                                    const float4 mu, int zp_sub, int lo) {
+  const uint64_t ones = f2_pack(1.0f, 1.0f), magic = f2_pack(MAGIC_F, MAGIC_F);
+  uint64_t t01 = f2_mul(f2_add(u2_pack(v0, v1), f2_pack(bd.x, bd.y)), f2_pack(mu.x, mu.y));
+  uint64_t t23 = f2_mul(f2_add(u2_pack(v2, v3), f2_pack(bd.z, bd.w)), f2_pack(mu.z, mu.w));
+  t01 = f2_fma(t01, ones, magic);
+  t23 = f2_fma(t23, ones, magic);
+  uint32_t r0, r1, r2, r3;
+  u2_unpack(t01, r0, r1);
+  u2_unpack(t23, r2, r3);
+  const int q0 = max((int)r0 + zp_sub, lo), q1 = max((int)r1 + zp_sub, lo);
+  const int q2 = max((int)r2 + zp_sub, lo), q3 = max((int)r3 + zp_sub, lo);
+  return pack_sat_u8(q1, q0, pack_sat_u8(q3, q2, 0u));
+}
+
 // 32 consecutive output channels of one pixel (one tcgen05.ld 32x32b.x32 worth): v -> 8 packed words.
 // cm: this pixel's border-class row of (MAGIC_BITS - corr), bd/mu: bdiv / mult, all at the chunk's first channel
 // (shared memory, or register arrays after inlining).  `fast` = layer flagged B200Q_RQ_BOUNDED.
@@ -427,6 +445,16 @@ __device__ __forceinline__ void tc_mma_i8(uint32_t tmem_d, uint64_t desc_a, uint
       "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// Same with fp16 operands and an fp32 accumulator (kind::f16, K = 16 per instruction).
+__device__ __forceinline__ void tc_mma_f16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                           uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
+      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 // Fill 32 lanes x 8 consecutive 32-bit columns with one value (thread t writes lane base_lane + t).
@@ -485,6 +513,14 @@ __host__ __device__ constexpr uint32_t make_idesc_i8(int m, int n) {
   return (2u << 4)                      // c_format = S32
          | (0u << 7)                    // a_format = UINT8
          | (1u << 10)                   // b_format = INT8
+         | (0u << 15) | (0u << 16)      // A, B K-major
+         | ((uint32_t)(n >> 3) << 17)   // N
+         | ((uint32_t)(m >> 4) << 24);  // M
+}
+// Instruction descriptor for kind::f16: D=f32, A=B=f16, both K-major, dense.
+__host__ __device__ constexpr uint32_t make_idesc_f16(int m, int n) {
+  return (1u << 4)                      // c_format = F32
+         | (0u << 7) | (0u << 10)       // a_format = b_format = F16
          | (0u << 15) | (0u << 16)      // A, B K-major
          | ((uint32_t)(n >> 3) << 17)   // N
          | ((uint32_t)(m >> 4) << 24);  // M

@@ -279,7 +279,7 @@ struct EpiTile {
   bool valid0, valid1;
 };
 
-template <bool CHECK, int NCH, class Consts>
+template <bool CHECK, bool F32ACC, int NCH, class Consts>
 __device__ __forceinline__ void epi_half(const uint32_t (&v)[2 * NCH], const EpiRegs<NCH>& K, const Consts& consts, int ch0,
                                          bool fast, int zp_out, int lo, uint8_t* out, int64_t stride_s, bool valid0,
                                          bool valid1) {
@@ -288,28 +288,39 @@ __device__ __forceinline__ void epi_half(const uint32_t (&v)[2 * NCH], const Epi
 #pragma unroll
   for (int s = 0; s < 2; ++s) {
     uint32_t packed[G];
-    uint32_t bad = 0;
-    if (fast) {
+    if constexpr (F32ACC) {  // exact fp32 accumulators, B200Q_RQ_BOUNDED constants: no range test, no fall-back
       const uint32_t* w = v + 2 * s;
-      packed[0] = epi_requant4<CHECK, 0>(w[0], w[1], w[4], w[5], K, zp_sub, lo, bad);
-      packed[1] = epi_requant4<CHECK, 4>(w[8], w[9], w[12], w[13], K, zp_sub, lo, bad);
-      if constexpr (G == 4) {
-        packed[2] = epi_requant4<CHECK, 8>(w[16], w[17], w[20], w[21], K, zp_sub, lo, bad);
-        packed[3] = epi_requant4<CHECK, 12>(w[24], w[25], w[28], w[29], K, zp_sub, lo, bad);
-      }
-    }
-    if (!fast || (CHECK && __any_sync(0xffffffffu, requant_magic_out_of_range(bad)))) {
 #pragma unroll
-      for (int g = 0; g < G; ++g) {
-        const uint32_t* w = v + 8 * g + 2 * s;
-        packed[g] = epi_requant4_exact(w[0], w[1], w[4], w[5], consts, ch0 + 4 * g, zp_out, lo);
+      for (int g = 0; g < G; ++g)
+        packed[g] = requant4_f32acc(w[8 * g], w[8 * g + 1], w[8 * g + 4], w[8 * g + 5],
+                                    make_float4(K.bd[4 * g], K.bd[4 * g + 1], K.bd[4 * g + 2], K.bd[4 * g + 3]),
+                                    make_float4(K.mu[4 * g], K.mu[4 * g + 1], K.mu[4 * g + 2], K.mu[4 * g + 3]), zp_sub, lo);
+    } else {
+      uint32_t bad = 0;
+      if (fast) {
+        const uint32_t* w = v + 2 * s;
+        packed[0] = epi_requant4<CHECK, 0>(w[0], w[1], w[4], w[5], K, zp_sub, lo, bad);
+        packed[1] = epi_requant4<CHECK, 4>(w[8], w[9], w[12], w[13], K, zp_sub, lo, bad);
+        if constexpr (G == 4) {
+          packed[2] = epi_requant4<CHECK, 8>(w[16], w[17], w[20], w[21], K, zp_sub, lo, bad);
+          packed[3] = epi_requant4<CHECK, 12>(w[24], w[25], w[28], w[29], K, zp_sub, lo, bad);
+        }
+      }
+      if (!fast || (CHECK && __any_sync(0xffffffffu, requant_magic_out_of_range(bad)))) {
+#pragma unroll
+        for (int g = 0; g < G; ++g) {
+          const uint32_t* w = v + 8 * g + 2 * s;
+          packed[g] = epi_requant4_exact(w[0], w[1], w[4], w[5], consts, ch0 + 4 * g, zp_out, lo);
+        }
       }
     }
     if (s == 0 ? valid0 : valid1) epi_store<G>(out + s * stride_s, packed);
   }
 }
 
-template <bool CHECK, int NCH, class Consts, class Next>
+// F32ACC: the accumulators are exact fp32 values of acc - corr (conv1_tc.cu) and every MMA of a tile starts from zero:
+// nothing to re-arm, so the slot goes back to the issuer as soon as half 1 has landed.
+template <bool CHECK, int NCH, bool F32ACC = false, class Consts, class Next>
 __device__ __forceinline__ void epi_pipeline(EpiRegs<NCH>& K, const Consts& consts, int ch0, bool fast, int zp_out, int lo,
                                              int64_t stride_s, int64_t stride_half, int lane, Next next) {
   constexpr int PARTW = 4 * NCH;
@@ -328,12 +339,18 @@ __device__ __forceinline__ void epi_pipeline(EpiRegs<NCH>& K, const Consts& cons
     // needs it three tiles later).
     tmem_ld_wait();                                     // half 0 has landed
     tmem_ld_frag<PARTW / 8>(cur.t_addr + HALF1, v1);    // half 1 in flight during the arithmetic of half 0
-    epi_half<CHECK>(v0, K, consts, ch0, fast, zp_out, lo, cur.out, stride_s, cur.valid0, cur.valid1);
+    epi_half<CHECK, F32ACC>(v0, K, consts, ch0, fast, zp_out, lo, cur.out, stride_s, cur.valid0, cur.valid1);
     tmem_ld_wait();                                     // half 1 has landed
+    if constexpr (F32ACC) {
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(cur.empty_bar);        // slot read: back to the MMA issuer
+    } else {
 #pragma unroll
-    for (int c = 0; c < PARTW; c += 16) {
-      tmem_st_fill_16x16(cur.t_addr + c, K.fill);
-      tmem_st_fill_16x16(cur.t_addr + HALF1 + c, K.fill);
+      for (int c = 0; c < PARTW; c += 16) {
+        tmem_st_fill_16x16(cur.t_addr + c, K.fill);
+        tmem_st_fill_16x16(cur.t_addr + HALF1 + c, K.fill);
+      }
     }
     EpiTile nxt;
     const bool have_next = next(nxt);
@@ -342,11 +359,13 @@ __device__ __forceinline__ void epi_pipeline(EpiRegs<NCH>& K, const Consts& cons
       tc_fence_after();
       tmem_ld_frag<PARTW / 8>(nxt.t_addr, v0);
     }
-    epi_half<CHECK>(v1, K, consts, ch0, fast, zp_out, lo, cur.out + stride_half, stride_s, cur.valid0, cur.valid1);
-    tmem_st_wait();
-    tc_fence_before();
-    __syncwarp();
-    if (lane == 0) mbar_arrive(cur.empty_bar);          // slot read and re-armed: back to the MMA issuer
+    epi_half<CHECK, F32ACC>(v1, K, consts, ch0, fast, zp_out, lo, cur.out + stride_half, stride_s, cur.valid0, cur.valid1);
+    if constexpr (!F32ACC) {
+      tmem_st_wait();
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(cur.empty_bar);        // slot read and re-armed: back to the MMA issuer
+    }
     cur = nxt;
     have = have_next;
   }
