@@ -20,6 +20,9 @@ import numpy as np
 import pytest
 import torch
 
+from tests._requant_regimes import (SAMPLE, _conv_batch, _conv_plan, _fc1_batch, _fc1_kernel, _plain_kernel_name,
+                                    _sample)
+
 pytestmark = pytest.mark.gpu
 
 CONVS = ("conv2", "conv3", "conv4", "conv5", "conv6")
@@ -29,8 +32,6 @@ CONV3_SIZES = ("nbi3_below", "nbi3_above")  # conv3: one image per band below 3 
 CONV1_SIZES = (1, 32, 33, 2048)  # conv1_kernel<C1_IN_F32, 1> up to CONV1_TINY_MAX_B = 32 images (simt.cu), conv1_tc_kernel above
 FC1_SIZES = ("1", "7", "narrow_last", "wide_first")
 NET_SIZES = ("1", "2", "pair_first", "nbi3_above", "fc1_wide")
-WHOLE = 160   # up to this many images every output is compared with the oracle; above it, a sample
-SAMPLE = 48
 
 
 def _cases():
@@ -46,80 +47,13 @@ CASES = _cases()
 
 
 # ---------------------------------------------------------------------------------------------- kernel selection
-def _geom(layer):
-    from convnet_quantization_b200.packing import CONV_GEOMETRY
-    return CONV_GEOMETRY[layer]  # (cin, cout, img)
-
-
-def _small_last(layer, sms):
-    """Largest batch for which ``b200q_conv3x3_tc`` runs the small-batch ``igemm_tc_kernel`` (N tile 64): the layer cut
-    into 128-pixel x 64-channel tiles fits in two waves of CTAs (37 / 74 / 74 / 148 / 148 on 148 SMs)."""
-    _, cout, img = _geom(layer)
-
-    def m_tiles(b):
-        return b * 8 if img == 32 else b * 2 if img == 16 else (b + 1) // 2
-
-    b = 3
-    while m_tiles(b + 1) * (cout // 64) <= 2 * sms:
-        b += 1
-    return b
-
-
-def _conv_batch(layer, size, sms):
-    last = _small_last(layer, sms)
-    first = last + 1
-    return {
-        "1": 1, "2": 2,                      # conv3x3_tiny_kernel (CONV_TINY_MAX_B = 2)
-        "3": 3, "small_last": last,          # igemm_tc_kernel<..., 64>
-        "band_first": first,                 # first batch on the band-resident kernels
-        # odd: the last CTA pair (conv2 + pool) or the last pair band (conv5 / conv6, 4 images) is partly empty
-        "band_odd": first + 1 if first % 2 == 0 else first + 2,
-        "nbi3_below": 3 * sms - 1, "nbi3_above": 3 * sms + 1,
-        "many": 9 * sms + 5,                 # every persistent CTA (pair) walks three or more bands
-    }[size]
-
-
-def _conv_plan(layer, pool, b, sms):
-    """(kernel-name pattern, images per band, bands in flight at once) that ``b200q_conv3x3_tc`` selects.  Patterns
-    are matched against demangled names with the spaces and ``(int)`` / ``(bool)`` casts removed."""
-    cin, cout, img = _geom(layer)
-    p = "true" if pool else "false"
-    if b <= 2:
-        return rf"conv3x3_tiny_kernel<{img},{cin},{cout},{p}>", 1, b
-    if b <= _small_last(layer, sms):
-        return rf"igemm_tc_kernel<{img},{cin},{cout},false,{p},(true|false),64>", 1, b
-    if layer == "conv2" and pool:
-        return r"conv_halo2_kernel<(true|false),8>", 2, sms // 2
-    if layer == "conv2":
-        return r"conv_halo_kernel<32,64,64,1,false,(true|false),8>", 1, sms
-    if layer == "conv3":
-        nbi = 1 if b < 3 * sms else 3
-        return rf"conv_halo_kernel<16,64,128,{nbi},false,(true|false),8>", nbi, sms
-    if layer == "conv4":
-        return rf"conv_halo_kernel<16,128,128,1,{p},(true|false),8>", 1, sms
-    return rf"conv_pair_kernel<{cin},{p},(true|false)>", 4, sms // 2
-
-
 def _conv1_kernel(b):
     return r"conv1_kernel<1,1>" if b <= 32 else r"conv1_tc_kernel<(true|false),false>"
-
-
-def _fc1_batch(size, sms):
-    narrow_last = 128 * (sms // 8)  # eight 64-column CTA tiles per 128 rows while they fit on the SMs
-    return {"1": 1, "7": 7, "narrow_last": narrow_last, "wide_first": narrow_last + 1}[size]
-
-
-def _fc1_kernel(b, sms):
-    return rf"igemm_tc_kernel<0,4096,512,false,false,true,{64 if b <= 128 * (sms // 8) else 0}>"
 
 
 def _net_batch(size, sms):
     return {"1": 1, "2": 2, "pair_first": sms + 1, "nbi3_above": 3 * sms + 1,
             "fc1_wide": _fc1_batch("wide_first", sms)}[size]
-
-
-def _plain_kernel_name(name):
-    return (name.replace(" ", "").replace("(int)", "").replace("(bool)0", "false").replace("(bool)1", "true"))
 
 
 # ---------------------------------------------------------------------------------------------- fixtures
@@ -179,22 +113,6 @@ def _oracle_conv(x_u8, L, pool):
     y = IO.conv2d_q(x_u8, L["in_scale"], L["in_zp"], L["w_int8"], L["w_scales"], L["bias"], L["out_scale"],
                     L["out_zp"], relu=False)
     return IO.max_pool2x2(y) if pool else y
-
-
-def _sample(b, band, walkers, seed):
-    """Every image up to ``WHOLE``; above, a fixed sample of at least ``SAMPLE`` images: the first and last two, both
-    sides of the first band boundary and of every boundary between rounds of the persistent CTAs, the last (maybe
-    partial) band, and seeded random images."""
-    if b <= WHOLE:
-        return np.arange(b)
-    idx = {0, 1, b - 2, b - 1, band - 1, band}
-    step = band * walkers
-    for lo in range(step, b, step):
-        idx.update((lo - 1, lo))
-    idx.update(range((b - 1) // band * band, b))
-    rest = np.setdiff1d(np.arange(b), np.fromiter(idx, dtype=np.int64))
-    fill = np.random.default_rng(seed).choice(rest, size=max(0, SAMPLE - len(idx)), replace=False)
-    return np.sort(np.concatenate([np.fromiter(idx, dtype=np.int64), fill]))
 
 
 def _assert_reaches_both_clamps(want, zp_out, what):
